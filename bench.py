@@ -405,6 +405,32 @@ def parity_on_tail(rec_gpu, text, guides, k, pam, synth, max_bases):
     return d
 
 
+DUMP_BYTES = 64_000_000        # --dump-outputs: at most this much array data per run
+
+
+def dump_arrays(out_dir, arrays, prefix=""):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def dump_records(out_dir, rec, prefix="", budget=DUMP_BYTES):
+    """--dump-outputs: the records a caller receives (REC_DT, emission order) as float64 columns <prefix>hits_<field>.npy, exact for
+    every field (u32 at most).  A list larger than the budget is replaced by a fixed sample (seed 0, indices sorted and written as
+    <prefix>hits_index.npy); <prefix>hits_total.npy holds the full record count either way."""
+    fields = ("guide", "flag", "contig", "pos", "mm")
+    n = len(rec)
+    cap = (budget - 4096) // (8 * (len(fields) + 1))
+    arrays = {"hits_total": [n]}
+    if n > cap:
+        idx = np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+        rec = rec[idx]
+        arrays["hits_index"] = idx
+    for f in fields:
+        arrays["hits_" + f] = rec[f]
+    dump_arrays(out_dir, arrays, prefix)
+
+
 def run_reference(args, cfg, world, rank):
     """--impl reference: the CPU oracle port on the host cores (SeqAn's bidir_mapping cannot be built here).  Same text
     (seeds, scale) and the same kind of sample as the GPU arm's cpu_baseline; the product library is never loaded."""
@@ -455,8 +481,9 @@ class Workload:
 
 
 def measure(V, ctx, text, guides, k, pam, first, words, steps, warmup, world, local, hits_buf, exchange, n_total_bases, ng, host_threads,
-            do_e2e=True, genome_words=None):
-    """value / value_cold / e2e (/ e2e_resident_genome) of one config on the given shard.  Returns a dict (rank 0: complete)."""
+            do_e2e=True, genome_words=None, keep_last=False):
+    """value / value_cold / e2e (/ e2e_resident_genome) of one config on the given shard.  Returns a dict (rank 0: complete);
+    keep_last: res["last_hits"] is a copy of the hit list of the last timed step of `value`."""
     from varscot_b200 import _lib
     res = {}
     units = float(ng) * n_total_bases                     # guide·bp per step over all ranks (strong: ONE text)
@@ -480,6 +507,8 @@ def measure(V, ctx, text, guides, k, pam, first, words, steps, warmup, world, lo
         barrier(world, local)
         ms = all_reduce(dev / steps, world, local, "MAX")
         digests[name] = hashlib.blake2b(hits.tobytes(), digest_size=16).hexdigest()      # the sorted list of this rank's shard
+        if keep_last and name == "warm":
+            res["last_hits"] = hits.copy()                                             # hits_buf is reused by the next scans
         res[name] = {"ms": ms, "value": units / (ms * 1e-3) / 1e9, "score_ms": score / steps, "resolve_ms": resolve / steps, "launches": launches,
                      "score_launches": int(st.score_launches), "blocks": int(st.n_blocks_fwd + st.n_blocks_rev), "index_build_ms": build_ms,
                      "bucketed": bool(all_reduce(float(st.index_reused == 2), world, local, "MIN")),
@@ -549,16 +578,36 @@ def measure(V, ctx, text, guides, k, pam, first, words, steps, warmup, world, lo
     return res, (rec, coll)
 
 
+def pick_canonical(h, key, idx):
+    """h[idx] (a copy) of a key-sorted hit list, except that hits of equal key (contig ids equal modulo 2^16, same guide, strand and
+    pos) arrive in no fixed order: a pick inside such a run takes the entry of the same rank in the run sorted by (contig, info)."""
+    out = h[idx]
+    tied = np.zeros(len(idx), dtype=bool)
+    tied[idx > 0] |= key[idx[idx > 0] - 1] == out["key"][idx > 0]
+    tied[idx < len(h) - 1] |= key[idx[idx < len(h) - 1] + 1] == out["key"][idx < len(h) - 1]
+    for i in np.nonzero(tied)[0]:
+        lo, hi = np.searchsorted(key, out["key"][i], "left"), np.searchsorted(key, out["key"][i], "right")
+        run = h[lo:hi]
+        out[i] = run[np.lexsort((run["info"], run["contig"]))[idx[i] - lo]]
+    return out
+
+
 def run_dense(args, cfg, V, synth, text, ctx, guides, first, words, world, rank, local, total_bases, all_cpus, t_gen, as_block=False):
-    """Config 5 (10 000 guides, k <= 8: ~1.9e9 hits): ONE pass through the end-to-end call with a sink.  The guides are scored in
-    super-chunks sized to the device hit buffer; every super-chunk is resolved + sorted on the device and handed to the host
-    (here: counted per guide, spot-checked for order), so host memory stays O(super-chunk) and no pass is repeated.
+    """Config 5 (10 000 guides, k <= 8: ~1.9e9 hits): passes through the end-to-end call with a sink, `--warmup` untimed ones, then
+    `--steps` timed ones (as_block: one timed pass).  The guides are scored in super-chunks sized to the device hit buffer; every
+    super-chunk is resolved + sorted on the device and handed to the host (here: counted per guide, spot-checked for order), so host
+    memory stays O(super-chunk).
     Standalone (`--config 5`) rank 0 prints the line; as_block (the `dense_cfg5` block of a multi-GPU default line) rank 0 returns it.
     The device part runs without a collective inside and never raises: a rank that fails says so in ONE all-reduce after it, so that
     no rank is left waiting for another (standalone: every rank then raises; block: the block is {"error": ...})."""
     desc, gbases, nvar, ng, k, pam, gseed = cfg
+    steps, warmup = (1, 0) if as_block else (args.steps, args.warmup)
+    dump = bool(args.dump_outputs) and not as_block
+    # --dump-outputs: per guide, up to `per_guide` of its delivered hits at evenly spaced ranks of its sorted list (the same entries
+    # whatever the super-chunks: a guide's hits always arrive in one delivery)
+    per_guide = max(1, (DUMP_BYTES // world - 4096 - 8 * ng) // (8 * 5 * ng))
     counts = np.zeros(ng, dtype=np.int64)
-    box = {"chunks": 0, "max_chunk": 0, "sorted": True, "host_s": 0.0}
+    box = {}
 
     def sink(h, lo, hi):
         """One delivery = the hits of guides [lo, hi), sorted; its key counts the guide from lo (bits 49..).  Per-guide counts come from
@@ -581,20 +630,36 @@ def run_dense(args, cfg, V, synth, text, ctx, guides, first, words, world, rank,
         counts[lo:hi] += c
         if box["chunks"] == 0:                                  # order spot check on the first delivery (a pass over its first 4 Mi entries)
             box["sorted"] = bool((np.diff(key[: 1 << 22].astype(np.int64)) >= 0).all())
+        if dump:
+            cs = c[nz]
+            m = np.minimum(cs, per_guide)
+            g = np.repeat(np.arange(len(nz)), m)
+            j = np.arange(int(m.sum())) - np.repeat(np.cumsum(m) - m, m)
+            box["sample"].append(pick_canonical(h, key, b[nz][g] + j * cs[g] // m[g]))
         box["chunks"] += 1; box["max_chunk"] = max(box["max_chunk"], len(h))
         box["host_s"] += time.perf_counter() - t
         return 0
+
+    def one_pass():
+        counts[:] = 0
+        box.update(chunks=0, max_chunk=0, sorted=True, host_s=0.0, sample=[])
+        t = time.perf_counter()
+        _, st_ = ctx.scan_resolved(guides, k, pam=pam, text=text, first_word=first, n_words=words, sink=sink)
+        return st_, (time.perf_counter() - t) * 1e3
 
     sampler = ClockSampler(local) if rank == 0 else None
     barrier(world, local)
     nv = 4
     err = None
     st = small = None
-    wall_ms = 0.0
-    t0_wall = time.time(); t0 = time.perf_counter()
+    dev_ms = wall_ms = 0.0
+    t0_wall = time.time()
     try:
-        _, st = ctx.scan_resolved(guides, k, pam=pam, text=text, first_word=first, n_words=words, sink=sink)
-        wall_ms = (time.perf_counter() - t0) * 1e3
+        for _ in range(warmup):
+            one_pass()
+        for _ in range(steps):
+            st, w = one_pass()
+            dev_ms += st.total_ms; wall_ms += w
         # verification scan of the first guides against the now resident index (same per-guide counts; parity with the oracle on a sample below)
         small, st_s = ctx.scan_resolved(guides[:nv], k, pam=pam, cap=1 << 22)
     except Exception as e:
@@ -607,19 +672,25 @@ def run_dense(args, cfg, V, synth, text, ctx, guides, first, words, world, rank,
         if not as_block:
             raise RuntimeError(msg)
         return {"error": msg} if rank == 0 else None
-    ms = all_reduce(float(st.total_ms), world, local, "MAX")
-    e_ms = all_reduce(wall_ms, world, local, "MAX")
+    ms = all_reduce(dev_ms / steps, world, local, "MAX")
+    e_ms = all_reduce(wall_ms / steps, world, local, "MAX")
     hits_total = all_reduce(float(counts.sum()), world, local, "SUM")
     same_counts = bool((np.bincount((small["info"] >> 8).astype(np.int64), minlength=nv) == counts[:nv]).all())
     same_counts = all_reduce(1.0 if same_counts else 0.0, world, local, "MIN") == 1.0
     redo_total = int(all_reduce(float(st.redo_chunks), world, local, "SUM"))
+    if dump:
+        s = np.concatenate(box["sample"]) if box["sample"] else np.zeros(0, V.LOC_DT)
+        dump_arrays(args.dump_outputs, {"hits_total": [counts.sum()], "hits_per_guide": counts, "hits_guide": s["info"] >> 8,
+                                        "hits_strand": (s["info"] >> 7) & 1, "hits_contig": s["contig"],
+                                        "hits_pos": s["key"] & np.uint64(0xFFFFFFFF), "hits_mm": s["info"] & 0x7F},
+                    f"rank{rank}_" if world > 1 else "")
     if rank != 0:
         return None
     units = float(ng) * total_bases
-    out = {"metric": "guide_Gbp_per_s", "value": units / (ms * 1e-3) / 1e9, "unit": "guide*Gbp/s", "n_gpus": world, "steps": 1, "warmup": 0,
+    out = {"metric": "guide_Gbp_per_s", "value": units / (ms * 1e-3) / 1e9, "unit": "guide*Gbp/s", "n_gpus": world, "steps": steps, "warmup": warmup,
            "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "u32 bit-sliced (LOP3)", "data": "synthetic",
            "config": config_dict(cfg, text.n_bases, text.n_contigs, "strong" if world > 1 else "single", args.scale),
-           "value_note": "config 5 is measured in ONE end-to-end pass (text from host buffers, hits to a host sink): value = CUDA-event time of that pass, e2e = its wall clock",
+           "value_note": "config 5 is measured in end-to-end passes (text from host buffers, hits to a host sink): value = mean CUDA-event time of the timed passes, e2e = their mean wall clock",
            "hits_per_step": int(hits_total), "hits_per_s": hits_total / (e_ms * 1e-3),
            "rank0": {"guide_passes": int(st.guide_passes), "redo": int(st.redo_chunks), "score_ms": float(st.score_ms), "extract_ms": float(st.extract_ms),
                      "resolve_sort_d2h_ms": float(st.resolve_ms), "sink_host_s": box["host_s"], "deliveries": box["chunks"], "largest_delivery": box["max_chunk"],
@@ -650,7 +721,8 @@ def run_dense_child(args, timeout_s):
     import signal
     env = {k_: v for k_, v in os.environ.items()
            if k_ not in ("RANK", "LOCAL_RANK", "WORLD_SIZE", "LOCAL_WORLD_SIZE", "GROUP_RANK", "ROLE_RANK", "MASTER_ADDR", "MASTER_PORT", "TORCHELASTIC_RUN_ID")}
-    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--config", "5", "--gpus", "1", "--scale", repr(args.scale)] + (["--no-cpu"] if args.no_cpu else [])
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--config", "5", "--gpus", "1", "--scale", repr(args.scale), "--steps", "1", "--warmup", "0"] + \
+        (["--no-cpu"] if args.no_cpu else [])
     t = time.perf_counter()
     p = subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env, start_new_session=True, cwd=ROOT)
     try:
@@ -729,8 +801,16 @@ def main():
     ap.add_argument("--no-dense", action="store_true", help="skip the dense_cfg5 block (config 5 in a child process; single-GPU default line only)")
     ap.add_argument("--cli", action="store_true", help="(default on the single-GPU config-3 line) the cli_e2e leg: the bidir_mapping executable from the .vsidx cache to the SAM file, wall clock")
     ap.add_argument("--no-cli", action="store_true", help="skip the cli_e2e leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of `value` computed as DIR/<name>.npy (float64, at most 64 MB; "
+                         "with several ranks every rank writes its shard's arrays as rank<r>_<name>.npy): its hit records in emission order; "
+                         "config 5 its per-guide hit counts and a fixed sample of the hits its sink received")
     args = ap.parse_args()
-    if args.warmup < 3 and args.impl == "ours":
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    if args.warmup < 3 and args.impl == "ours" and args.config != 5:      # (config 5's passes need no warm-up of a resident index)
         args.warmup = 3
     cfg = list(CONFIGS[args.config])
     if args.guides:
@@ -802,8 +882,12 @@ def main():
     time.sleep(0.15)
     t0_wall = time.time()
     res, merged = measure(V, ctx, text, guides, k, pam, first, words, args.steps, args.warmup, world, local, hits_buf, exchange,
-                          total_bases, ng, host_threads, do_e2e=not args.no_e2e)
+                          total_bases, ng, host_threads, do_e2e=not args.no_e2e, keep_last=bool(args.dump_outputs))
     clocks = sampler.stop(t0_wall, time.time()) if sampler else None
+    if args.dump_outputs:
+        rec_last, _ = V.merge_resolved([res.pop("last_hits")], threads=host_threads)
+        dump_records(args.dump_outputs, rec_last, f"rank{rank}_" if world > 1 else "", DUMP_BYTES // world)
+        del rec_last
 
     # ---- resident genome: only the variant segments (and the guides) travel per call ---------------------------
     e2e_rg = None

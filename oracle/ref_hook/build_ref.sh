@@ -1,6 +1,6 @@
 #!/bin/bash
-# oracle/ref_hook/build_ref.sh — TEST INFRASTRUCTURE.  Derives two artefacts from the reference tree where it lies
-# (default /root/reference), outputs ONLY into oracle/_ref/ (git-ignored; it travels to the GPU box with gpurun):
+# oracle/ref_hook/build_ref.sh <VARSCOT checkout> — TEST INFRASTRUCTURE.  Derives two artefacts from a checkout of the upstream
+# VARSCOT repository, outputs ONLY into oracle/_ref/ (git-ignored):
 #
 #  1. oracle/_ref/VARSCOT           the reference's own driver script (VARSCOT_pipeline/VARSCOT) with its two stray
 #                                   `then` lines removed (`else` followed by `then` at :297-298 and :312-313 makes bash
@@ -9,12 +9,12 @@
 #  2. oracle/_ref/bidir_mapping,    the TRUE reference read mapper, built with the reference's own CMake project
 #     oracle/_ref/bidir_index       (VARSCOT_pipeline/read_mapping/CMakeLists.txt) — ONLY when a SeqAn 2.4.0rc2 checkout
 #                                   exists at $SEQAN_DIR or <reference>/VARSCOT_pipeline/lib/seqan (the reference clones it
-#                                   at docker-build time, Dockerfile:41; it is absent from this image, so today this
-#                                   step reports "unbuildable" and parity stays unpinned).  The day it is supplied,
+#                                   at docker-build time, Dockerfile:41; without it this step reports "unbuildable"
+#                                   and parity stays unpinned).  The day it is supplied,
 #                                   tools/diff_against_ref.sh diffs the oracle and the CUDA mapper against it.
 set -u
 HERE="$(cd "$(dirname "$0")" && pwd)"
-REF="${1:-/root/reference}"
+REF="${1:?usage: build_ref.sh <checkout of the upstream VARSCOT repository>}"
 OUT="$HERE/../_ref"
 [ -d "$REF/VARSCOT_pipeline" ] || { echo "build_ref: no reference tree at $REF (nothing to do)"; exit 0; }
 mkdir -p "$OUT"

@@ -1,9 +1,9 @@
-"""Generates the committed golden fixtures under tests/golden/ (run in the build container).
+"""Generates the committed golden fixtures under tests/golden/:  python tests/golden/make_golden.py [<VARSCOT checkout>]
 
 * ref_guides.fa : the 16 real guides the reference ships as inputs for this path
   (workflow/guideseq-data/guideseqOntargets.fasta, workflow/siteseq-data/siteseqOntargets.fasta) —
   input data only; the reference holds NO expected outputs for bidir_mapping (its one golden SAM is a
-  git-LFS pointer), so parity stays "unpinned".
+  git-LFS pointer), so parity stays "unpinned".  Rewritten only when a checkout of upstream VARSCOT is given.
 * case_*.json   : small seeded cases with the ORACLE's records and SAM text; they pin the oracle against
   accidental change and give the GPU tests an oracle-independent file to compare with.
 """
@@ -20,13 +20,11 @@ sys.path.insert(0, ROOT)
 from oracle import oracle as O          # noqa: E402
 from tests.util import make_case        # noqa: E402
 
-REF = "/root/reference/workflow"
 
-
-def ref_guides():
+def ref_guides(workflow):
     out = []
     for f in ("guideseq-data/guideseqOntargets.fasta", "siteseq-data/siteseqOntargets.fasta"):
-        out.append(open(os.path.join(REF, f)).read())
+        out.append(open(os.path.join(workflow, f)).read())
     open(os.path.join(HERE, "ref_guides.fa"), "w").write("".join(out))
 
 
@@ -41,8 +39,8 @@ def dump_case(name, case, md_style=O.MD_SEQAN):
 
 
 if __name__ == "__main__":
-    if os.path.isdir(REF):
-        ref_guides()
+    if len(sys.argv) > 1:
+        ref_guides(os.path.join(sys.argv[1], "workflow"))
     dump_case("case_k4", make_case(seed=1001, contig_lens=[6000, 45, 45, 23, 0, 22, 3000], n_guides=4, k=4))
     dump_case("case_k6_pamAG", make_case(seed=1002, contig_lens=[8000, 45, 2000], n_guides=5, k=6, pam="AG"))
     dump_case("case_k8", make_case(seed=1003, contig_lens=[5000, 46, 47, 1000], n_guides=3, k=8))

@@ -57,6 +57,63 @@ def test_gpu_arm_shared_memory_handover_and_dense_mode():
     assert d["parity"]["diff"] == 0 and d["rank0"]["first_delivery_sorted"] and d["e2e"]["value"] > 0
 
 
+@pytest.mark.gpu
+def test_gpu_arm_dump_outputs_equal_oracle(tmp_path):
+    """--dump-outputs: the records of the last timed scan, as written by the GPU arm, are the oracle's records of the same text."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "3", "--scale", "0.001", "--steps", "2", "--warmup", "3",
+                        "--no-cpu", "--no-e2e", "--no-target", "--no-dense", "--no-cli", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    from oracle import oracle as O
+    core = bench.load_synth_core()
+    text = core.build_workload(3_100_000_000, 5_000_000, 0.001)
+    exp = O.map_guides(core.unpack_codes(text, 0, text.n_bases), text.offsets, core.synth_guides(13, 100), 6)
+    assert len(exp.guide) > 0 and np.load(tmp_path / "hits_total.npy").tolist() == [len(exp.guide)]
+    for f in ("guide", "flag", "contig", "pos", "mm"):
+        assert (np.load(tmp_path / f"hits_{f}.npy") == getattr(exp, f)).all(), f
+
+
+def test_dump_records_samples_a_large_list_the_same_way_every_time(tmp_path):
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    from varscot_b200.mapper import REC_DT
+    rec = np.zeros(1000, dtype=REC_DT)
+    rec["guide"] = np.arange(1000) % 7; rec["contig"] = np.arange(1000) // 3; rec["pos"] = 4_000_000_000 - np.arange(1000); rec["mm"] = 2
+    budget = 4096 + 48 * 100                                     # room for 100 records (5 columns + their indices)
+    for d in ("a", "b"):
+        bench.dump_records(str(tmp_path / d), rec, "rank1_", budget)
+    idx = np.load(tmp_path / "a" / "rank1_hits_index.npy")
+    assert len(idx) == 100 and (np.diff(idx) > 0).all() and np.load(tmp_path / "a" / "rank1_hits_total.npy").tolist() == [1000]
+    for f in ("guide", "flag", "contig", "pos", "mm"):
+        a = np.load(tmp_path / "a" / f"rank1_hits_{f}.npy")
+        assert (a == rec[f][idx.astype(np.int64)]).all() and (a == np.load(tmp_path / "b" / f"rank1_hits_{f}.npy")).all()
+    assert sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir()) <= budget
+
+
+def test_pick_canonical_ignores_the_order_of_equal_keys():
+    """Hits of equal key may arrive in either order: the picks (and so config 5's dumped sample) must not depend on it."""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    from varscot_b200.mapper import LOC_DT
+    h = np.zeros(12, dtype=LOC_DT)
+    h["key"] = [1, 2, 5, 5, 5, 7, 8, 8, 9, 10, 11, 11]
+    h["contig"] = np.arange(12) + 70000
+    h["info"] = np.arange(12)
+    other = h.copy()
+    other[2:5] = h[2:5][::-1]                                    # the same list with its runs of equal keys in another order
+    other[6:8] = h[6:8][::-1]
+    other[10:12] = h[10:12][::-1]
+    idx = np.array([0, 2, 3, 4, 7, 9, 11])
+    a, b = bench.pick_canonical(h, h["key"], idx), bench.pick_canonical(other, other["key"], idx)
+    assert (a == b).all() and sorted(a["contig"].tolist()) == sorted(h["contig"][idx].tolist())
+
+
 def test_static_evidence_helpers():
     """The bench line quotes ncu's pipe loads and DRAM bytes from the committed captures and reduces `nvidia-smi topo -m` to one
     entry: both parsers against the files under profiles/ (no GPU, no nvidia-smi needed)."""

@@ -150,6 +150,7 @@ def _install_fakes(world, rank, port):
 
 
 def _run(rank, world, port, argv, q):
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""                    # no device for the run nor its child processes, on a GPU machine too
     os.environ["MASTER_PORT"] = str(port)                      # (HostExchange names its segments after it)
     os.environ["TORCHELASTIC_RUN_ID"] = f"dry{port}"
     if world == 1:
@@ -209,6 +210,45 @@ def test_bench_dense_block_failure_on_one_rank_costs_only_the_block(monkeypatch)
     d = _spawn(2, ["--gpus", "2", "--config", "3", "--scale", "0.0002", "--steps", "2", "--warmup", "3"])
     assert "error" in d["dense_cfg5"] and "another rank" in d["dense_cfg5"]["error"]
     assert d["parity"]["diff"] == 0 and d["e2e"]["value"] > 0 and d["target_cfg4"]["parity"]["diff"] == 0
+
+
+def test_bench_dump_outputs_are_the_records_of_the_timed_scan(tmp_path):
+    """--dump-outputs writes the records of the last timed step of `value` as float64 columns; the stand-in answers with the oracle's
+    records, so they must be the oracle's records of the whole text, in emission order."""
+    _spawn(1, ["--config", "3", "--scale", "0.0002", "--steps", "2", "--warmup", "3", "--no-cpu", "--no-target", "--no-dense", "--no-cli",
+               "--dump-outputs", str(tmp_path)])
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle import oracle as O
+    core = bench.load_synth_core()
+    text = core.build_workload(3_100_000_000, 5_000_000, 0.0002)
+    r = O.map_guides(core.unpack_codes(text, 0, text.n_bases), text.offsets, core.synth_guides(13, 100), 6)
+    assert len(r.guide) > 0 and np.load(tmp_path / "hits_total.npy").tolist() == [len(r.guide)]
+    assert not (tmp_path / "hits_index.npy").exists()
+    for f in ("guide", "flag", "contig", "pos", "mm"):
+        a = np.load(tmp_path / f"hits_{f}.npy")
+        assert a.dtype == np.float64 and (a == getattr(r, f)).all(), f
+
+
+def test_bench_config5_steps_and_dump_outputs(tmp_path):
+    """Config 5 times --steps passes after --warmup ones; --dump-outputs writes its per-guide counts and, per guide, evenly spaced
+    entries of what the sink received: here (oracle records) a subset of the oracle's hits, of the size the byte budget allows."""
+    d = _spawn(1, ["--config", "5", "--scale", "0.0005", "--guides", "200", "--steps", "3", "--warmup", "1", "--no-cpu",
+                   "--dump-outputs", str(tmp_path)])
+    assert d["steps"] == 3 and d["warmup"] == 1 and d["hits_per_step"] > 100
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle import oracle as O
+    core = bench.load_synth_core()
+    text = core.build_workload(3_100_000_000, 5_000_000, 0.0005)
+    r = O.map_guides(core.unpack_codes(text, 0, text.n_bases), text.offsets, core.synth_guides(15, 200), 8)
+    counts = np.bincount(r.guide, minlength=200)
+    assert (np.load(tmp_path / "hits_per_guide.npy") == counts).all() and np.load(tmp_path / "hits_total.npy").tolist() == [len(r.guide)]
+    got = {f: np.load(tmp_path / f"hits_{f}.npy").astype(np.int64) for f in ("guide", "strand", "contig", "pos", "mm")}
+    per_guide = (bench.DUMP_BYTES - 4096 - 8 * 200) // (8 * 5 * 200)
+    assert (np.bincount(got["guide"], minlength=200) == np.minimum(counts, per_guide)).all()
+    exp = set(zip(r.guide.tolist(), ((r.flag & 16) >> 4).tolist(), r.contig.tolist(), r.pos.tolist(), r.mm.tolist()))
+    assert set(zip(*(got[f].tolist() for f in ("guide", "strand", "contig", "pos", "mm")))) <= exp
 
 
 @pytest.mark.parametrize("world", [1, 2])

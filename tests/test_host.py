@@ -6,6 +6,7 @@ import json
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -47,11 +48,16 @@ def test_product_never_touches_the_oracle():
 
 
 def test_no_device_fails_loudly():
-    if V.device_count() > 0:
-        pytest.skip("a GPU is present")
-    with pytest.raises(V.VarscotError) as e:
-        V.ScanContext(0)
-    assert e.value.code == _lib.VS_ERR_NODEVICE
+    """In a child process that sees no device (so that the test runs on a GPU machine too)."""
+    code = ("import sys; sys.path.insert(0, sys.argv[1])\n"
+            "import pytest, varscot_b200 as V\n"
+            "from varscot_b200 import _lib\n"
+            "assert V.device_count() == 0\n"
+            "with pytest.raises(V.VarscotError) as e:\n"
+            "    V.ScanContext(0)\n"
+            "assert e.value.code == _lib.VS_ERR_NODEVICE\n")
+    r = subprocess.run([sys.executable, "-c", code, ROOT], capture_output=True, text=True, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stderr
 
 
 def _expected_masks(codes, off):
@@ -350,9 +356,9 @@ def test_cli_contract_exit_codes(tmp_path):
     # wrong guide length is refused
     write_guides(str(tmp_path / "bad.fa"), ["a"], ["ACGT"])
     assert run_cli("bidir_mapping", "-G", g, "-I", tmp_path / "idx", "-R", tmp_path / "bad.fa", "-M", 4, "-O", tmp_path / "o.sam").returncode == 1
-    if V.device_count() == 0:
-        x = run_cli("bidir_mapping", *base, "-M", 4)
-        assert x.returncode == 1 and "no usable CUDA device" in x.stderr and "Reads loaded (total: 2)." in x.stdout
+    x = subprocess.run([os.path.join(BIN, "bidir_mapping"), *map(str, base), "-M", "4"], capture_output=True, text=True,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))              # no device visible, on a GPU machine too
+    assert x.returncode == 1 and "no usable CUDA device" in x.stderr and "Reads loaded (total: 2)." in x.stdout
 
 
 def test_resolve_hits_threads_agree():
