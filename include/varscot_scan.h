@@ -155,8 +155,18 @@ const char *vs_last_error(const vs_ctx *ctx);   /* ctx may be NULL: last error o
 /* words per pipeline chunk (default 4 Mi words = 128 Mi bases); tests shrink it to cross chunk borders */
 int  vs_ctx_set_chunk_words(vs_ctx *ctx, uint64_t chunk_words);
 
+/* Limits.  A text of any length is accepted; a contig holds at most 2^32 bases (positions inside a contig are 32-bit).
+ * Positions inside a context are 32-bit and relative to the shard's origin: 0 — they are global — for every shard of a
+ * text within 4 Gbases and for a shard that ends at least 32 bases below 2^32; the shard's first base otherwise.  Such a
+ * shard (one that reaches beyond 2^32 - 32 in a text longer than 4 Gbases) holds at most VS_MAX_SHARD_WORDS words.
+ * vs_scan_resolved, vs_map_records and the executables serve every text; the unordered calls (vs_scan, vs_scan_text,
+ * vs_scan_fetch, vs_map_packed) report global 32-bit positions and return VS_ERR_ARG beyond that domain (a text longer
+ * than 4 Gbases, or a resident shard whose origin is not 0). */
+#define VS_MAX_SHARD_WORDS ((1ull << 27) - 256)      /* 2^32 - 8192 bases, a whole number of 256-word tiles */
+
 /* Make words [first_word, first_word + n_words) of the text resident on the device (+ one halo word of bases).
- * Window STARTS in those words are owned by this context; hit positions are global (32 * first_word + local). */
+ * Window STARTS in those words are owned by this context; hit positions are 32 * first_word + local - origin (global
+ * for every text within 4 Gbases, see the limits above). */
 int vs_text_upload(vs_ctx *ctx, const vs_text_view *text, uint64_t first_word, uint64_t n_words);
 
 /* page-locked host memory for fast uploads / hit downloads */
@@ -164,7 +174,7 @@ void *vs_host_alloc(size_t bytes);
 void  vs_host_free(void *p);
 
 typedef struct {
-    uint32_t pos;    /* global start position in the concatenated text */
+    uint32_t pos;    /* start position in the concatenated text (global: the unordered calls serve texts within 4 Gbases) */
     uint32_t info;   /* guide << 8 | strand << 7 | mm  (strand 1 = reverse pass, flag bit 16) */
 } vs_hit;
 
@@ -232,7 +242,8 @@ int vs_host_unregister(void *p);
 
 /* Convenience used by the executables and bindings: shard a packed text by word ranges over the given
  * devices (devices == NULL or n_devices == 0 -> device 0; one host thread + one context per device, no
- * collective), scan, and return all hits unordered in a malloc'd array (release with vs_free). */
+ * collective), scan, and return all hits unordered in a malloc'd array (release with vs_free).
+ * Texts within 4 Gbases only (VS_ERR_ARG beyond: use vs_map_records). */
 int vs_map_packed(const vs_text_view *text, const uint8_t *guides, uint32_t n_guides,
                   int k, int extra_pam, const int *devices, int n_devices,
                   vs_hit **hits, uint64_t *n_hits, vs_scan_stats *stats);
@@ -266,7 +277,9 @@ int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t *counts, in
                       vs_record *out, uint64_t *key16_collisions, int n_threads);
 
 /* The whole mapping step of the executables: shard, scan with device-side resolution, merge; records in emission order
- * in a malloc'd array (release with vs_free). */
+ * in a malloc'd array (release with vs_free).  A text within 4 Gbases gets one shard per device (vs_shard_bounds); a
+ * longer one max(n_devices, ceil(n_words / VS_MAX_SHARD_WORDS)) shards rounded up to a multiple of n_devices, which every
+ * device scans one after the other. */
 int vs_map_records(const vs_text_view *text, const uint8_t *guides, uint32_t n_guides,
                    int k, int extra_pam, const int *devices, int n_devices, int n_threads,
                    vs_record **records, uint64_t *n_records, uint64_t *key16_collisions, vs_scan_stats *stats);

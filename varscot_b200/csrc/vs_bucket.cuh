@@ -160,7 +160,7 @@ k_bucket_scatter(const uint32_t *__restrict__ planes_f, const uint32_t *__restri
                  const uint32_t *__restrict__ pos_r, const unsigned long long *__restrict__ rng_all, PamParams pp,
                  unsigned long long *__restrict__ cursor, uint32_t *__restrict__ out_f, uint32_t *__restrict__ out_r, uint64_t cap_f, uint64_t cap_r)
 {
-    VS_BK_SMEM(h);                                // uint32_t h[BK_N]: first the CTA's count per bucket, then the first slot of its range (slots fit 32 bits: <= 4 G bases)
+    VS_BK_SMEM(h);                                // uint32_t h[BK_N]: first the CTA's count per bucket, then the first slot of its range (slots fit 32 bits: a shard holds < 4 G bases)
     const int strand = blockIdx.y;
     const unsigned long long n_blocks = rng_all[2 + strand];
     const unsigned long long cta0 = (unsigned long long)blockIdx.x * BKB_THREADS;
@@ -200,8 +200,8 @@ k_bucket_scatter(const uint32_t *__restrict__ planes_f, const uint32_t *__restri
 
 // k_bucket_gather: one thread per block of the bucketed store: the 23-base windows of its 32 positions are gathered from
 // the resident text (funnel shifts over two words of each plane), transposed to the bit-sliced block layout of k_extract
-// (48 words at plane_index) and written; padding slots get an empty valid bit.  first_base = global position of the
-// shard's word 0.
+// (48 words at plane_index) and written; padding slots get an empty valid bit.  first_base = position of the shard's word 0
+// relative to the shard's origin, as the positions in `pos`.
 __global__ void __launch_bounds__(64)
 k_bucket_gather(const vs_bases *__restrict__ B, const vs_masks *__restrict__ M, uint64_t first_base, const uint32_t *__restrict__ pos,
                 unsigned long long n_blocks, uint32_t *__restrict__ planes)

@@ -188,6 +188,17 @@ bool parse_int(const std::string &s, long &v)
 
 Opt *find_opt(std::vector<Opt> &opts, char s) { for (auto &o : opts) if (o.s == s) return &o; return nullptr; }
 
+// positions inside a sequence are 32-bit (SAM POS, vs_record.pos): true if every contig holds at most 2^32 bases
+bool contigs_fit(const char *prog, const vs_text_view &v)
+{
+    for (uint32_t c = 0; c < v.n_contigs; ++c)
+        if (v.contig_off[c + 1] - v.contig_off[c] > (1ull << 32)) {
+            fprintf(stderr, "%s: sequence %u has more than 4 giga bases (2^32); a single sequence may not be longer\n", prog, c);
+            return false;
+        }
+    return true;
+}
+
 // Several mapper processes run concurrently (VARSCOT:321-322 runs two, parallel.py:17 up to 48 pipelines).  Each process
 // takes an advisory lock (flock on /tmp/varscot_b200_gpu<i>.lock, held until it exits) on the first free device,
 // starting at pid % n: concurrent processes land on different GPUs as long as there are free ones, and share them
@@ -237,7 +248,7 @@ extern "C" int vs_bidir_index_main(int argc, char **argv)
     };
     int pr = parse_args(prog, argc, argv, opts,
                         "VARSCOT - Index Creation (B200 build): packs a multi-sequence FASTA (Dna5: A, C, G, T, N) into the "
-                        "bit-sliced text the GPU scan reads. At most 4 giga bases in total.");
+                        "bit-sliced text the GPU scan reads. Any total length; each sequence at most 4 giga bases (2^32).");
     if (pr == 2) return 0;
     if (pr == 1) return 1;
     std::string genome = find_opt(opts, 'G')->value, index = find_opt(opts, 'I')->value;
@@ -247,7 +258,7 @@ extern "C" int vs_bidir_index_main(int argc, char **argv)
     const auto t0 = std::chrono::steady_clock::now();
     if (!pack_fasta(genome, t, true, err)) { fprintf(stderr, "%s: %s\n", prog, err.c_str()); return 1; }
     const auto t1 = std::chrono::steady_clock::now();
-    if (t.v.n_bases > (1ull << 32)) { fprintf(stderr, "%s: the FASTA file may not contain more than 4 giga bases in total\n", prog); return 1; }
+    if (!contigs_fit(prog, t.v)) return 1;
     printf("Number of sequences: %u\n", t.v.n_contigs);
     fflush(stdout);
     if (vs_text_save(index.c_str(), &t.v) != VS_OK) {
@@ -282,7 +293,8 @@ extern "C" int vs_bidir_mapping_main(int argc, char **argv)
     };
     int pr = parse_args(prog, argc, argv, opts,
                         "Read mapper for CRISPR-Cas9 off-targets (B200 build). Only supports Dna4 reads (everything else than ACGT "
-                        "will be converted to A). All reads must have the same length (23).");
+                        "will be converted to A). All reads must have the same length (23). Texts of any total length; each sequence at "
+                        "most 4 giga bases (2^32).");
     if (pr == 2) return 0;
     if (pr == 1) return 1;
     long mism = 0, threads = 1;
@@ -360,7 +372,7 @@ extern "C" int vs_bidir_mapping_main(int argc, char **argv)
         fprintf(stderr, "%s: note: no packed text at %s.vsidx (%s); packing %s now\n", prog, index.c_str(), vs_last_error(nullptr), genome.c_str());
         if (!pack_fasta(genome, t, true, err)) { fprintf(stderr, "%s: %s\n", prog, err.c_str()); return 1; }
     }
-    if (t.v.n_bases > (1ull << 32)) { fprintf(stderr, "%s: text exceeds 4 giga bases\n", prog); return 1; }
+    if (!contigs_fit(prog, t.v)) return 1;
     printf("Index loaded.\n");
     fflush(stdout);
     const auto tm1 = std::chrono::steady_clock::now();

@@ -746,11 +746,13 @@ extern "C" int vs_format_sam(const vs_record *r, const char *qname, const char *
 // sharding across devices: contiguous word ranges, no collective, hits concatenated on the host
 namespace vs {
 
+constexpr uint64_t SHARD_TILE = 256;      // shard starts are tile-aligned
+
 std::vector<uint64_t> shard_bounds(uint64_t n_words, int n)
 {
     if (n < 1) n = 1;
     std::vector<uint64_t> b((size_t)n + 1, 0);
-    const uint64_t tile = 256;   // keep shard starts tile-aligned
+    const uint64_t tile = SHARD_TILE;
     uint64_t tiles = (n_words + tile - 1) / tile;
     for (int i = 0; i <= n; ++i) {
         uint64_t t = tiles * (uint64_t)i / (uint64_t)n;
@@ -760,11 +762,26 @@ std::vector<uint64_t> shard_bounds(uint64_t n_words, int n)
     return b;
 }
 
-static void add_stats(vs_scan_stats *agg, const vs_scan_stats &s)
+std::vector<uint64_t> shard_plan(uint64_t n_words, int n_devices)
 {
-    agg->upload_ms = std::max(agg->upload_ms, s.upload_ms); agg->extract_ms = std::max(agg->extract_ms, s.extract_ms);
-    agg->score_ms = std::max(agg->score_ms, s.score_ms); agg->total_ms = std::max(agg->total_ms, s.total_ms);
-    agg->resolve_ms = std::max(agg->resolve_ms, s.resolve_ms);
+    if (n_devices < 1) n_devices = 1;
+    uint64_t n = (uint64_t)n_devices;
+    if (n_words * 32 > (1ull << 32)) {
+        const uint64_t tiles = (n_words + SHARD_TILE - 1) / SHARD_TILE, per = VS_MAX_SHARD_WORDS / SHARD_TILE;
+        n = std::max<uint64_t>(n, (tiles + per - 1) / per);            // no shard gets more than `per` tiles
+        n = (n + n_devices - 1) / n_devices * n_devices;
+    }
+    return shard_bounds(n_words, (int)n);
+}
+
+// times of scans that ran at the same time on different devices: the slowest; of shards one device scanned one after
+// the other (`sequential`): the sum
+static void add_stats(vs_scan_stats *agg, const vs_scan_stats &s, bool sequential = false)
+{
+    const auto t = [sequential](float a, float b) { return sequential ? a + b : std::max(a, b); };
+    agg->upload_ms = t(agg->upload_ms, s.upload_ms); agg->extract_ms = t(agg->extract_ms, s.extract_ms);
+    agg->score_ms = t(agg->score_ms, s.score_ms); agg->total_ms = t(agg->total_ms, s.total_ms);
+    agg->resolve_ms = t(agg->resolve_ms, s.resolve_ms);
     agg->n_cand_fwd += s.n_cand_fwd; agg->n_cand_rev += s.n_cand_rev;
     agg->n_blocks_fwd += s.n_blocks_fwd; agg->n_blocks_rev += s.n_blocks_rev;
     agg->n_hits += s.n_hits; agg->launches += s.launches; agg->score_launches += s.score_launches;
@@ -772,24 +789,29 @@ static void add_stats(vs_scan_stats *agg, const vs_scan_stats &s)
     agg->guide_passes = std::max(agg->guide_passes, s.guide_passes);
 }
 
-// One host thread + one context per device, each scanning its word range of the text; `run(i, ctx, w0, n)` does the scan.
+// One host thread + one context per device; the shards of the plan b (a multiple of the device count) are dealt out in
+// contiguous runs, and each device scans its run one shard after the other on its context.  `run(s, ctx, w0, n)` scans
+// shard s.
 template <class Run>
-static int for_each_shard(const vs_text_view &text, const std::vector<int> &devices_in, vs_scan_stats *agg, std::string &err, Run run)
+static int for_each_shard(const std::vector<uint64_t> &b, const std::vector<int> &devices, vs_scan_stats *agg, std::string &err, Run run)
 {
-    std::vector<int> devices = devices_in;
-    if (devices.empty()) devices.push_back(0);
-    const int nd = (int)devices.size();
-    std::vector<uint64_t> b = shard_bounds(text.n_words, nd);
+    const int nd = (int)devices.size(), per = (int)(b.size() - 1) / nd;
     std::vector<int> rc((size_t)nd, VS_OK);
     std::vector<std::string> errs((size_t)nd);
     std::vector<vs_scan_stats> st((size_t)nd);
     auto work = [&](int i) {
         vs_ctx *ctx = nullptr;
         memset(&st[(size_t)i], 0, sizeof(vs_scan_stats));
-        uint64_t w0 = b[(size_t)i], w1 = b[(size_t)i + 1];
-        if (w1 <= w0) return;
-        int r = vs_ctx_create(devices[(size_t)i], &ctx);
-        if (r == VS_OK) r = run(i, ctx, w0, w1 - w0, &st[(size_t)i]);
+        int r = VS_OK;
+        for (int s = i * per; s < (i + 1) * per && r == VS_OK; ++s) {
+            const uint64_t w0 = b[(size_t)s], w1 = b[(size_t)s + 1];
+            if (w1 <= w0) continue;
+            if (!ctx) r = vs_ctx_create(devices[(size_t)i], &ctx);
+            vs_scan_stats one;
+            memset(&one, 0, sizeof(one));
+            if (r == VS_OK) r = run(s, ctx, w0, w1 - w0, &one);
+            if (r == VS_OK) add_stats(&st[(size_t)i], one, true);
+        }
         if (r != VS_OK) errs[(size_t)i] = vs_last_error(ctx);
         rc[(size_t)i] = r;
         vs_ctx_destroy(ctx);
@@ -808,13 +830,16 @@ static int for_each_shard(const vs_text_view &text, const std::vector<int> &devi
     return VS_OK;
 }
 
+static std::vector<int> or_device0(const std::vector<int> &devices) { return devices.empty() ? std::vector<int>{0} : devices; }
+
 int scan_text_sharded(const vs_text_view &text, const std::vector<int> &devices_in,
                       const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
                       std::vector<vs_hit> &hits, vs_scan_stats *agg, std::string &err)
 {
-    const size_t nd = devices_in.empty() ? 1 : devices_in.size();
-    std::vector<std::vector<vs_hit>> part(nd);
-    int rc = for_each_shard(text, devices_in, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
+    const std::vector<int> devices = or_device0(devices_in);
+    const std::vector<uint64_t> b = shard_plan(text.n_words, (int)devices.size());
+    std::vector<std::vector<vs_hit>> part(b.size() - 1);
+    int rc = for_each_shard(b, devices, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
         uint64_t cnt = 0;
         std::vector<vs_hit> &h = part[(size_t)i];
         h.resize(1u << 16);
@@ -838,8 +863,9 @@ int scan_text_sharded_resolved(const vs_text_view &text, const std::vector<int> 
                                const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
                                std::vector<std::vector<vs_loc_hit>> &lists, vs_scan_stats *agg, std::string &err)
 {
-    const size_t nd = devices_in.empty() ? 1 : devices_in.size();
-    lists.assign(nd, {});
+    const std::vector<int> devices = or_device0(devices_in);
+    const std::vector<uint64_t> b = shard_plan(text.n_words, (int)devices.size());
+    lists.assign(b.size() - 1, {});
     struct Sink {
         static int put(void *user, const vs_loc_hit *h, uint64_t n, uint32_t, uint32_t)
         {
@@ -848,7 +874,7 @@ int scan_text_sharded_resolved(const vs_text_view &text, const std::vector<int> 
             return 0;
         }
     };
-    return for_each_shard(text, devices_in, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
+    return for_each_shard(b, devices, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
         uint64_t cnt = 0;
         vs_ctx_set_option(ctx, VS_OPT_KEEP_INDEX, 0);
         return vs_scan_resolved(ctx, &text, w0, n, guides, n_guides, k, extra_pam, nullptr, 0, &cnt, &Sink::put, &lists[(size_t)i], st);
@@ -863,6 +889,10 @@ extern "C" int vs_map_packed(const vs_text_view *text, const uint8_t *guides, ui
 {
     if (!hits || !n_hits || !text) return VS_ERR_ARG;
     *hits = nullptr; *n_hits = 0;
+    if (text->n_words * 32 > (1ull << 32)) {
+        vs_set_last_error("vs_map_packed: unordered hits carry global 32-bit positions, which end at 4 Gbases of text: use vs_map_records");
+        return VS_ERR_ARG;
+    }
     std::vector<int> dev;
     for (int i = 0; i < n_devices && devices; ++i) dev.push_back(devices[i]);
     std::vector<vs_hit> h;

@@ -107,7 +107,8 @@ __device__ __forceinline__ void transpose32(uint32_t (&a)[32])
 constexpr int EX_THREADS   = 64;                  // threads per extraction CTA
 constexpr int EX_MAX_WORDS = 256;                 // words per tile (<=); the host picks the tile so that it holds ~60 blocks
 
-// k_extract: one 64-thread CTA per tile of `tile_words` words.
+// k_extract: one 64-thread CTA per tile of `tile_words` words.  global_base = position of device word 0 (relative to the
+// shard's position origin: the 32-bit positions it writes are global - origin).
 //   phase 1 (bit-parallel, 32 starts per word): candidate masks per strand -> shared memory + exclusive rank prefix;
 //   phase 2 (one THREAD per 32-candidate block): walk the masks from the block's first candidate, gather the 23-base
 //            windows (funnel shifts on the staged planes), transpose 32 x 23 bits twice in registers, write
@@ -677,7 +678,8 @@ k_extract_mark(unsigned long long *cnt, unsigned long long *rng, unsigned long l
 // k_contig_starts_*: the start positions of the contigs that overlap the shard, from the shard's contig-end plane
 // (em, one bit per base, set on the last base of a contig): starts[0] = first_start (given by the host: the contig that
 // holds the shard's first base), starts[r + 1] = position after the r-th end bit.  Three steps: bits per tile of
-// CS_TILE words, exclusive scan of the tile counts (one CTA), scatter.
+// CS_TILE words, exclusive scan of the tile counts (one CTA), scatter.  Positions are relative to the shard's origin
+// (first_base = position of device word 0); first_start may lie before the origin and is then stored modulo 2^32.
 constexpr int CS_TILE = 2048;              // words per CTA of 256 threads (8 per thread)
 __global__ void __launch_bounds__(256)
 k_contig_starts_count(const uint32_t *__restrict__ em, uint64_t n_words, uint32_t *__restrict__ tile_cnt)
@@ -739,8 +741,11 @@ k_contig_starts_scatter(const uint32_t *__restrict__ em, uint64_t n_words, const
     }
 }
 
-// k_resolve_hits: hit {global position, info} -> sort key + payload.  The contig is the last one whose start is <= the
+// k_resolve_hits: hit {position, info} -> sort key + payload.  The contig is the last one whose start is <= the
 // position (binary search over the shard's n_starts contig starts; contig id = first_contig + index);
+// positions and starts are relative to the shard's origin.  starts[0] is never compared (every probe has mid >= 1): the
+// first contig may begin before the origin, its start is then stored modulo 2^32, and pos - starts[0] wraps to the exact
+// position in the contig (a contig holds at most 2^32 bases).
 //   key = (guide - guide_lo) << 49 | strand << 48 | (contig & 0xFFFF) << 32 | pos in contig     (the std::map order of
 //         bidir_mapping.cpp:13,154 inside the pass order of :285-295)
 //   val = contig << 32 | info

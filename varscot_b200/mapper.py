@@ -285,7 +285,9 @@ class ScanContext:
         return hits[: n.value]
 
     def scan(self, guides: np.ndarray, k: int, pam=None, cap: int = 1 << 20, out: np.ndarray | None = None):
-        """Scan the resident text (vs_scan). Returns (hits structured array, ScanStats). Hits are unordered."""
+        """Scan the resident text (vs_scan). Returns (hits structured array, ScanStats). Hits are unordered, at global 32-bit
+        positions: a resident shard of a text beyond 4 Gbases whose positions are shard-relative raises VarscotError
+        (VS_ERR_ARG); scan_resolved serves it."""
         g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
         pc = pam if isinstance(pam, int) else pam_code(pam)
         hits = out if out is not None else np.zeros(cap, dtype=HIT_DT)
@@ -297,7 +299,8 @@ class ScanContext:
 
     def scan_text(self, text: PackedText, guides: np.ndarray, k: int, pam=None, first_word: int = 0, n_words: int | None = None,
                   cap: int = 1 << 20, out: np.ndarray | None = None, use_sparse: bool = True, use_source: bool = True):
-        """Upload (overlapped, chunk by chunk) and scan in one call (vs_scan_text): the end-to-end path."""
+        """Upload (overlapped, chunk by chunk) and scan in one call (vs_scan_text): the end-to-end path.  Texts within 4 Gbases
+        only (hits at global 32-bit positions); beyond, VarscotError (VS_ERR_ARG): use scan_resolved or map_records."""
         if n_words is None:
             n_words = text.n_words - first_word
         g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
@@ -364,7 +367,8 @@ def device_count() -> int:
 
 
 def map_packed(text: PackedText, guides: np.ndarray, k: int, pam=None, devices=None):
-    """vs_map_packed: shard over devices, scan, return (hits, stats)."""
+    """vs_map_packed: shard over devices, scan, return (hits, stats).  Texts within 4 Gbases only (hits at global 32-bit
+    positions); beyond, VarscotError (VS_ERR_ARG): use map_records."""
     L = _lib.lib()
     g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
     dev = np.asarray(devices if devices else [0], dtype=np.int32)
@@ -381,7 +385,8 @@ def map_packed(text: PackedText, guides: np.ndarray, k: int, pam=None, devices=N
 
 def map_records(text: PackedText, guides: np.ndarray, k: int, pam=None, devices=None, threads: int = 1):
     """vs_map_records: what the bidir_mapping executable runs — shard over devices, scan with device-side hit resolution,
-    merge.  Returns (records in emission order, key16_collisions, stats)."""
+    merge.  Texts of any length: beyond 4 Gbases every device scans one or more shards of at most VS_MAX_SHARD_WORDS words
+    one after the other.  Returns (records in emission order, key16_collisions, stats)."""
     L = _lib.lib()
     g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
     dev = np.asarray(devices if devices else [0], dtype=np.int32)
