@@ -19,6 +19,7 @@
  *                                  seed search + verify delegate, for both strands
  * vs_scan_resolved                 the same + the std::map<TOccType,..> order of :13,154 (contig lookup and sort on the device)
  * vs_resolve_hits / vs_merge_resolved  bidir_mapping.cpp:154,164-187  std::map order + primary/secondary flags
+ * vs_mapper_*                      bidir_mapping.cpp:268-295 with the index kept open across many guide sets
  * vs_md_string / vs_format_sam     bidir_mapping.cpp:111-123 getMDString + tags; :177-187 write(.., Sam())
  * vs_bidir_index_main              bidir_index.cpp:10-52   main (argv contract)
  * vs_bidir_mapping_main            bidir_mapping.cpp:190-312 main (argv contract, stdout lines, exit codes)
@@ -283,6 +284,32 @@ int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t *counts, in
 int vs_map_records(const vs_text_view *text, const uint8_t *guides, uint32_t n_guides,
                    int k, int extra_pam, const int *devices, int n_devices, int n_threads,
                    vs_record **records, uint64_t *n_records, uint64_t *key16_collisions, vs_scan_stats *stats);
+
+/* ---- resident mapper ------------------------------------------------------------------------------------------
+ * vs_map_records with the text kept in HBM between calls: a caller that maps many guide sets against one genome (a guide
+ * screen, a service, a batch that keeps the reference loaded) pays the upload once, the extraction of the candidate index
+ * once per PAM set, and from the second call on scores the bucketed index wherever VS_OPT_BUCKET_INDEX's default policy
+ * builds it.  Beyond 4 Gbases every device keeps all of its shards resident at once. */
+typedef struct vs_mapper vs_mapper;
+/* Shard `text` over the devices exactly as vs_map_records does (vs_shard_bounds within 4 Gbases, one shard per device;
+ * several per device beyond) and upload every shard to a context of its own that keeps its candidate index (devices == NULL
+ * or n_devices == 0 -> device 0).  The view's host buffers are read during this call only and may be released afterwards;
+ * the view must carry contig_off.  Before anything is uploaded, the device memory every device's shards will need (text,
+ * masks, the plain and the bucketed candidate store at the densest PAM set, the scan scratch of every context) is compared
+ * with its free memory: VS_ERR_NOMEM, with the bytes needed and free in vs_last_error(NULL), when it does not fit.  A failed
+ * upload releases everything and names the device and the shard.  VS_ERR_NODEVICE without a device. */
+int  vs_mapper_create(const vs_text_view *text, const int *devices, int n_devices, vs_mapper **out);
+/* Same arguments and results as vs_map_records, against the resident shards: records in emission order (malloc'd, release
+ * with vs_free).  The first call, and the first after a change of extra_pam, extracts the candidate index from the resident
+ * text; later calls score it.  stats: index_reused is the least over the shards (2 only when every shard scored its bucketed
+ * index), index_build_ms sums over a device's shards and takes the slowest device.  An argument error returns VS_ERR_ARG and
+ * leaves the resident shards and indexes as they were; so does a call made while another one runs on the same mapper. */
+int  vs_mapper_map(vs_mapper *m, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam, int n_threads,
+                   vs_record **records, uint64_t *n_records, uint64_t *key16_collisions, vs_scan_stats *stats);
+/* shards held; bytes of device memory the mapper's contexts hold now, and the create-time estimate (all devices; an upper
+ * bound for scans that keep up to 16 Mi hits per shard and pass, of up to 4096 guides) */
+int  vs_mapper_info(const vs_mapper *m, uint32_t *n_shards, uint64_t *device_bytes, uint64_t *planned_bytes);
+void vs_mapper_destroy(vs_mapper *m);
 
 #define VS_MD_SEQAN 0
 #define VS_MD_SAMTOOLS 1

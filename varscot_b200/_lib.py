@@ -70,6 +70,7 @@ EXPORTS = [
     "vs_ctx_create", "vs_ctx_destroy", "vs_last_error", "vs_ctx_set_chunk_words", "vs_text_upload", "vs_host_alloc",
     "vs_host_free", "vs_host_register", "vs_host_unregister", "vs_ctx_set_option", "vs_index_drop", "vs_scan", "vs_scan_text", "vs_scan_fetch",
     "vs_scan_resolved", "vs_merge_resolved", "vs_map_packed", "vs_shard_bounds", "vs_resolve_hits", "vs_resolve_hits_mt",
+    "vs_mapper_create", "vs_mapper_map", "vs_mapper_info", "vs_mapper_destroy",
     "vs_md_string", "vs_format_sam", "vs_bidir_index_main", "vs_bidir_mapping_main", "vs_vcf_loader_main", "vs_fasta_writer_main", "vs_bam_merger_main", "vs_bam_merger_ref_only_main", "vs_measure_int_peaks",
 ]
 
@@ -121,6 +122,10 @@ def lib():
     L.vs_host_unregister.argtypes = [vp]
     L.vs_map_packed.argtypes = [C.POINTER(TextView), vp, u32, i32, i32, vp, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(ScanStats)]
     L.vs_shard_bounds.argtypes = [u64, i32, vp]
+    L.vs_mapper_create.argtypes = [C.POINTER(TextView), vp, i32, C.POINTER(vp)]
+    L.vs_mapper_map.argtypes = [vp, vp, u32, i32, i32, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(ScanStats)]
+    L.vs_mapper_info.argtypes = [vp, C.POINTER(u32), C.POINTER(u64), C.POINTER(u64)]
+    L.vs_mapper_destroy.argtypes = [vp]
     L.vs_resolve_hits.argtypes = [vp, u64, vp, u32, vp, C.POINTER(u64)]
     L.vs_resolve_hits_mt.argtypes = [vp, u64, vp, u32, vp, C.POINTER(u64), i32]
     L.vs_md_string.argtypes = [vp, u64, vp, i32, i32, C.c_char_p]

@@ -218,6 +218,79 @@ extern "C" int vs_index_drop(vs_ctx *ctx)
     return VS_OK;
 }
 
+// ---- device memory accounting (vs_mapper) -----------------------------------------------------------------------------
+constexpr uint64_t BLOCK_BYTES = BLK_WORDS * 4 + 32 * 4;            // one block of 32 candidates: planes + positions
+
+uint64_t vs::ctx_device_bytes(const vs_ctx *ctx)
+{
+    if (!ctx) return 0;
+    uint64_t b = ctx->words_cap * (sizeof(vs_bases) + sizeof(vs_masks)) + ctx->sparse_cap * sizeof(vs_mask_entry);
+    b += ctx->planes_cap * (2 * sizeof(uint32_t) + 1) + ctx->dense_cap + ctx->runs_cap * sizeof(vs_plane_run);
+    b += (ctx->cstart_cap + ctx->tilecnt_cap + 1) * sizeof(uint32_t);
+    if (ctx->d_cnt) b += (4 + 4 * (ctx->cnt_chunks + 1) + 4 + 4) * sizeof(unsigned long long);
+    b += 2 * ctx->blocks_cap * BLOCK_BYTES + (ctx->bk_cap[0] + ctx->bk_cap[1]) * BLOCK_BYTES;
+    if (ctx->d_bk_ctl) b += (2 * BK_N + 2 * BK_N + 2 * (BK_N + 1)) * sizeof(unsigned long long);
+    if (ctx->d_cls) b += 2ull * BK_N * BK_CLS * sizeof(uint32_t);
+    b += (ctx->perm_cap + ctx->gkey_cap + ctx->pat_cap) * sizeof(uint16_t);
+    b += ctx->hits_cap * sizeof(vs_hit) + ctx->loc_cap * (4 * 8 + sizeof(vs_loc_hit)) + ctx->sort_tmp_bytes;
+    return b;
+}
+
+// Candidate store of a shard, blocks per strand: the expected n_pam / 16 candidates per strand and base, + 15 %, + one partial
+// block per extraction tile and per chunk (what scan_engine allocates before the first extraction)
+static uint32_t default_tile_words(int n_pam) { return (uint32_t)(60.0 * 16.0 / (2.0 * n_pam)) & ~7u; }
+
+static uint64_t cand_store_blocks(uint64_t n_words, int n_pam, uint32_t tile_words, uint64_t n_chunks)
+{
+    const uint64_t tiles = (n_words + tile_words - 1) / tile_words;
+    const uint64_t est = (uint64_t)((double)n_words * n_pam / 16.0 * 1.15) + tiles + 64ull * n_chunks + 256;
+    return (est + BLK_GROUP - 1) / BLK_GROUP * BLK_GROUP;
+}
+
+uint64_t vs::resident_shard_bytes(const ShardShape &s, uint64_t text_words, int n_pam)
+{
+    const uint64_t w = s.words, n_chunks = (w + DEFAULT_CHUNK_WORDS - 1) / DEFAULT_CHUNK_WORDS + 3;
+    // text: bases + window masks, both planes + code bytes of the contig-end plane, coded-block flags of the whole text, the
+    // staged runs (or sparse mask entries) of the upload, contig starts and their tile counts, counters
+    uint64_t b = (w + 1) * (sizeof(vs_bases) + sizeof(vs_masks) + 2 * sizeof(uint32_t) + 1) + (text_words + VS_EM_BLOCK) / VS_EM_BLOCK;
+    b += (s.staged + 4 * n_chunks + 16) * sizeof(vs_plane_run);
+    b += (s.contigs + 4 + (w + CS_TILE - 1) / CS_TILE + 1 + 1) * sizeof(uint32_t);
+    b += (4 + 4 * (n_chunks + 8 + 1) + 4 + 4) * sizeof(unsigned long long);
+    // candidate store of both strands, and its bucketed form: every bucket padded to whole batches, + 1/64 + one batch
+    const uint64_t plain = cand_store_blocks(w, n_pam, default_tile_words(n_pam), n_chunks);
+    const uint64_t bucketed = plain + (uint64_t)BK_N * SC_NB;
+    b += 2 * plain * BLOCK_BYTES + 2 * (bucketed + bucketed / 64 + SC_NB) * BLOCK_BYTES;
+    b += (2 * BK_N + 2 * BK_N + 2 * (BK_N + 1)) * sizeof(unsigned long long) + 2ull * BK_N * BK_CLS * sizeof(uint32_t);
+    // scan scratch: hit buffer, resolution and sort buffers, pattern and class tables
+    b += RESIDENT_SCRATCH_HITS * sizeof(vs_hit) + (RESIDENT_SCRATCH_HITS + RESIDENT_SCRATCH_HITS / 8) * (4 * 8 + sizeof(vs_loc_hit)) + (64ull << 20);
+    b += 2ull * RESIDENT_SCRATCH_GUIDES * (PAT_STRIDE + 1 + BK_N) * sizeof(uint16_t);
+    return b;
+}
+
+int vs::resident_plan_check(const std::vector<ShardShape> &shards, uint64_t text_words, const std::vector<uint64_t> &free_bytes,
+                            std::vector<uint64_t> &need)
+{
+    const size_t nd = free_bytes.size(), per = nd ? shards.size() / nd : 0;
+    need.assign(nd, 0);
+    int first_short = -1;
+    for (size_t i = 0; i < nd; ++i) {
+        for (size_t s = i * per; s < (i + 1) * per; ++s)
+            if (shards[s].words) need[i] += resident_shard_bytes(shards[s], text_words, 3);
+        if (need[i] > free_bytes[i] && first_short < 0) first_short = (int)i;
+    }
+    return first_short;
+}
+
+int vs::device_free_bytes(int device, uint64_t *free_bytes)
+{
+    vs_ctx *ctx = nullptr;
+    size_t f = 0, t = 0;
+    CK(cudaSetDevice(device));
+    CK(cudaMemGetInfo(&f, &t));
+    *free_bytes = f;
+    return VS_OK;
+}
+
 extern "C" int vs_host_register(void *p, size_t bytes)
 {
     if (!p || !bytes) return VS_ERR_ARG;
@@ -831,7 +904,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
     const std::vector<uint64_t> plan = chunk_plan(n_words, chunk_words, src != nullptr);
     const uint32_t n_chunks = (uint32_t)(plan.size() - 1);
     // tile size: about 60 blocks (both strands) per 64-thread CTA at the expected PAM density pp.n / 16 per strand
-    uint32_t tile_words = (uint32_t)(60.0 * 16.0 / (2.0 * pp.n)) & ~7u;
+    uint32_t tile_words = default_tile_words(pp.n);
     if (const char *e = getenv("VARSCOT_TILE_WORDS")) tile_words = (uint32_t)atoi(e);      // tuning knob
     if (tile_words > (uint32_t)EX_MAX_WORDS) tile_words = EX_MAX_WORDS;
     if (tile_words < 8) tile_words = 8;
@@ -891,10 +964,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
     const bool reuse = !src && ctx->idx_valid && ctx->idx_pam == q.extra_pam;
     if (!reuse) {
         ctx->idx_valid = false; ctx->bk_valid = false;
-        const uint64_t tiles = (n_words + tile_words - 1) / tile_words;
-        uint64_t est = (uint64_t)((double)n_words * pp.n / 16.0 * 1.15) + tiles + 64ull * n_chunks + 256;
-        est = (est + BLK_GROUP - 1) / BLK_GROUP * BLK_GROUP;
-        if ((r = ensure_blocks(est)) != VS_OK) return r;
+        if ((r = ensure_blocks(cand_store_blocks(n_words, pp.n, tile_words, n_chunks))) != VS_OK) return r;
     }
     // a resident index that is scanned again gets its bucketed form (built once; this scan pays for it)
     bool use_bk = false;

@@ -775,46 +775,51 @@ std::vector<uint64_t> shard_plan(uint64_t n_words, int n_devices)
 }
 
 // times of scans that ran at the same time on different devices: the slowest; of shards one device scanned one after
-// the other (`sequential`): the sum
-static void add_stats(vs_scan_stats *agg, const vs_scan_stats &s, bool sequential = false)
+// the other (`sequential`): the sum.  index_reused is the least over the shards (`first`: s is the first one added).
+static void add_stats(vs_scan_stats *agg, const vs_scan_stats &s, bool sequential, bool first)
 {
     const auto t = [sequential](float a, float b) { return sequential ? a + b : std::max(a, b); };
     agg->upload_ms = t(agg->upload_ms, s.upload_ms); agg->extract_ms = t(agg->extract_ms, s.extract_ms);
     agg->score_ms = t(agg->score_ms, s.score_ms); agg->total_ms = t(agg->total_ms, s.total_ms);
-    agg->resolve_ms = t(agg->resolve_ms, s.resolve_ms);
+    agg->resolve_ms = t(agg->resolve_ms, s.resolve_ms); agg->index_build_ms = t(agg->index_build_ms, s.index_build_ms);
     agg->n_cand_fwd += s.n_cand_fwd; agg->n_cand_rev += s.n_cand_rev;
     agg->n_blocks_fwd += s.n_blocks_fwd; agg->n_blocks_rev += s.n_blocks_rev;
     agg->n_hits += s.n_hits; agg->launches += s.launches; agg->score_launches += s.score_launches;
     agg->h2d_bytes += s.h2d_bytes; agg->d2h_bytes += s.d2h_bytes; agg->n_chunks += s.n_chunks; agg->redo_chunks += s.redo_chunks;
     agg->guide_passes = std::max(agg->guide_passes, s.guide_passes);
+    agg->index_reused = first ? s.index_reused : std::min(agg->index_reused, s.index_reused);
 }
 
-// One host thread + one context per device; the shards of the plan b (a multiple of the device count) are dealt out in
-// contiguous runs, and each device scans its run one shard after the other on its context.  `run(s, ctx, w0, n)` scans
-// shard s.
+// One host thread per device; the shards of the plan b (a multiple of the device count) are dealt out in contiguous runs,
+// and each device runs its shards one after the other.  `run(s, ctx, w0, n, stats)` handles shard s on ctx.
+//   shard_ctx == nullptr: every device gets one context for the call, shared by its shards and destroyed at the end;
+//   otherwise (*shard_ctx)[s] is shard s's own context: created on the shard's device when it is null, and kept.
+// An empty shard is skipped and gets no context.
 template <class Run>
-static int for_each_shard(const std::vector<uint64_t> &b, const std::vector<int> &devices, vs_scan_stats *agg, std::string &err, Run run)
+static int for_each_shard(const std::vector<uint64_t> &b, const std::vector<int> &devices, std::vector<vs_ctx *> *shard_ctx,
+                          vs_scan_stats *agg, std::string &err, Run run)
 {
     const int nd = (int)devices.size(), per = (int)(b.size() - 1) / nd;
-    std::vector<int> rc((size_t)nd, VS_OK);
+    std::vector<int> rc((size_t)nd, VS_OK), failed((size_t)nd, -1), ran((size_t)nd, 0);
     std::vector<std::string> errs((size_t)nd);
     std::vector<vs_scan_stats> st((size_t)nd);
     auto work = [&](int i) {
-        vs_ctx *ctx = nullptr;
+        vs_ctx *own = nullptr;
         memset(&st[(size_t)i], 0, sizeof(vs_scan_stats));
         int r = VS_OK;
         for (int s = i * per; s < (i + 1) * per && r == VS_OK; ++s) {
             const uint64_t w0 = b[(size_t)s], w1 = b[(size_t)s + 1];
             if (w1 <= w0) continue;
+            vs_ctx *&ctx = shard_ctx ? (*shard_ctx)[(size_t)s] : own;
             if (!ctx) r = vs_ctx_create(devices[(size_t)i], &ctx);
             vs_scan_stats one;
             memset(&one, 0, sizeof(one));
             if (r == VS_OK) r = run(s, ctx, w0, w1 - w0, &one);
-            if (r == VS_OK) add_stats(&st[(size_t)i], one, true);
+            if (r == VS_OK) add_stats(&st[(size_t)i], one, true, ran[(size_t)i]++ == 0);
+            else { errs[(size_t)i] = vs_last_error(ctx); failed[(size_t)i] = s; }
         }
-        if (r != VS_OK) errs[(size_t)i] = vs_last_error(ctx);
         rc[(size_t)i] = r;
-        vs_ctx_destroy(ctx);
+        vs_ctx_destroy(own);
     };
     if (nd == 1) work(0);
     else {
@@ -823,10 +828,40 @@ static int for_each_shard(const std::vector<uint64_t> &b, const std::vector<int>
         for (auto &t : th) t.join();
     }
     if (agg) memset(agg, 0, sizeof(*agg));
+    bool first = true;
     for (int i = 0; i < nd; ++i) {
-        if (rc[(size_t)i] != VS_OK) { err = "device " + std::to_string(devices[(size_t)i]) + ": " + errs[(size_t)i]; return rc[(size_t)i]; }
-        if (agg) add_stats(agg, st[(size_t)i]);
+        if (rc[(size_t)i] != VS_OK) {
+            err = "device " + std::to_string(devices[(size_t)i]) + (shard_ctx ? ", shard " + std::to_string(failed[(size_t)i]) : std::string()) + ": " + errs[(size_t)i];
+            return rc[(size_t)i];
+        }
+        if (agg && ran[(size_t)i]) { add_stats(agg, st[(size_t)i], false, first); first = false; }
     }
+    return VS_OK;
+}
+
+// the sink of vs_scan_resolved that appends every super-chunk to a std::vector<vs_loc_hit>
+static int append_sink(void *user, const vs_loc_hit *h, uint64_t n, uint32_t, uint32_t)
+{
+    auto *v = static_cast<std::vector<vs_loc_hit> *>(user);
+    try { v->insert(v->end(), h, h + n); } catch (...) { return 1; }
+    return 0;
+}
+
+// the shard lists of vs_scan_resolved -> records in emission order (malloc'd; NULL when there are none)
+static int merge_lists(const std::vector<std::vector<vs_loc_hit>> &lists, int n_threads, vs_record **records, uint64_t *n_records,
+                       uint64_t *key16_collisions)
+{
+    std::vector<const vs_loc_hit *> ptr;
+    std::vector<uint64_t> cnt;
+    uint64_t total = 0;
+    for (auto &l : lists) { ptr.push_back(l.data()); cnt.push_back(l.size()); total += l.size(); }
+    if (key16_collisions) *key16_collisions = 0;
+    if (total == 0) return VS_OK;
+    vs_record *o = (vs_record *)malloc(total * sizeof(vs_record));
+    if (!o) return VS_ERR_NOMEM;
+    const int rc = vs_merge_resolved(ptr.data(), cnt.data(), (int)ptr.size(), o, key16_collisions, n_threads);
+    if (rc != VS_OK) { free(o); return rc; }
+    *records = o; *n_records = total;
     return VS_OK;
 }
 
@@ -839,7 +874,7 @@ int scan_text_sharded(const vs_text_view &text, const std::vector<int> &devices_
     const std::vector<int> devices = or_device0(devices_in);
     const std::vector<uint64_t> b = shard_plan(text.n_words, (int)devices.size());
     std::vector<std::vector<vs_hit>> part(b.size() - 1);
-    int rc = for_each_shard(b, devices, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
+    int rc = for_each_shard(b, devices, nullptr, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
         uint64_t cnt = 0;
         std::vector<vs_hit> &h = part[(size_t)i];
         h.resize(1u << 16);
@@ -866,22 +901,141 @@ int scan_text_sharded_resolved(const vs_text_view &text, const std::vector<int> 
     const std::vector<int> devices = or_device0(devices_in);
     const std::vector<uint64_t> b = shard_plan(text.n_words, (int)devices.size());
     lists.assign(b.size() - 1, {});
-    struct Sink {
-        static int put(void *user, const vs_loc_hit *h, uint64_t n, uint32_t, uint32_t)
-        {
-            auto *v = static_cast<std::vector<vs_loc_hit> *>(user);
-            try { v->insert(v->end(), h, h + n); } catch (...) { return 1; }
-            return 0;
-        }
-    };
-    return for_each_shard(b, devices, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
+    return for_each_shard(b, devices, nullptr, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
         uint64_t cnt = 0;
         vs_ctx_set_option(ctx, VS_OPT_KEEP_INDEX, 0);
-        return vs_scan_resolved(ctx, &text, w0, n, guides, n_guides, k, extra_pam, nullptr, 0, &cnt, &Sink::put, &lists[(size_t)i], st);
+        return vs_scan_resolved(ctx, &text, w0, n, guides, n_guides, k, extra_pam, nullptr, 0, &cnt, &append_sink, &lists[(size_t)i], st);
     });
 }
 
 }  // namespace vs
+
+// ------------------------------------------------------------------------------------------------
+// resident mapper: the shards of vs_map_records, each on a context of its own that keeps its text and candidate indexes
+struct vs_mapper {
+    std::vector<int> devices;
+    std::vector<uint64_t> bounds;          // vs::shard_plan
+    std::vector<vs_ctx *> ctx;             // per shard; null for an empty shard
+    uint64_t planned_bytes = 0;
+    std::atomic<bool> busy{false};
+};
+
+extern "C" void vs_mapper_destroy(vs_mapper *m)
+{
+    if (!m) return;
+    for (vs_ctx *c : m->ctx) vs_ctx_destroy(c);
+    delete m;
+}
+
+extern "C" int vs_mapper_create(const vs_text_view *text, const int *devices, int n_devices, vs_mapper **out)
+{
+    if (out) *out = nullptr;
+    if (!out || !text || (!devices && n_devices > 0) || n_devices < 0) { vs_set_last_error("vs_mapper_create: NULL argument"); return VS_ERR_ARG; }
+    if (!text->contig_off || text->n_contigs == 0) { vs_set_last_error("vs_mapper_create: the text view carries no contig offsets"); return VS_ERR_ARG; }
+    const int n_visible = vs_device_count();
+    if (n_visible <= 0) { vs_set_last_error("vs_mapper_create: no CUDA device visible (this library has no CPU fallback)"); return VS_ERR_NODEVICE; }
+    std::vector<int> dev;
+    for (int i = 0; i < n_devices; ++i) {
+        if (devices[i] < 0 || devices[i] >= n_visible) { vs_set_last_error(("vs_mapper_create: device " + std::to_string(devices[i]) + " does not exist").c_str()); return VS_ERR_ARG; }
+        dev.push_back(devices[i]);
+    }
+    if (dev.empty()) dev.push_back(0);
+    const int nd = (int)dev.size();
+    const std::vector<uint64_t> b = vs::shard_plan(text->n_words, nd);
+    const size_t n_shards = b.size() - 1;
+    // what every shard will hold: its words, the contigs that overlap it, the entries its upload stages
+    std::vector<vs::ShardShape> shape(n_shards);
+    const uint64_t *ob = text->contig_off, *oe = text->contig_off + text->n_contigs + 1;
+    const bool src = text->em_code && text->em_dense;
+    auto in_range = [](const auto *v, uint64_t n, uint64_t lo, uint64_t hi, auto end_of) {
+        const auto *a = std::partition_point(v, v + n, [&](const auto &x) { return end_of(x) <= lo; });
+        return (uint64_t)(std::partition_point(a, v + n, [&](const auto &x) { return (uint64_t)x.word < hi; }) - a);
+    };
+    const auto run_end = [](const vs_plane_run &r) { return (uint64_t)r.word + r.count; };
+    const auto entry_end = [](const vs_mask_entry &e) { return (uint64_t)e.word + 1; };
+    for (size_t s = 0; s < n_shards; ++s) {
+        const uint64_t w0 = b[s], w1 = b[s + 1];
+        if (w1 <= w0) continue;
+        const uint64_t c0 = (uint64_t)(std::upper_bound(ob, oe, w0 * 32) - ob), c1 = (uint64_t)(std::upper_bound(ob, oe, w1 * 32) - ob);
+        shape[s].words = w1 - w0;
+        shape[s].contigs = c1 - c0 + 1;
+        if (src) shape[s].staged = in_range(text->nm_runs, text->n_nm_runs, w0, w1 + 1, run_end) + in_range(text->em_runs, text->n_em_runs, w0, w1 + 1, run_end);
+        else if (text->sparse) shape[s].staged = in_range(text->sparse, text->n_sparse, w0, w1, entry_end);
+    }
+    // device memory check before anything is uploaded
+    std::vector<uint64_t> free_b((size_t)nd, 0), need;
+    std::vector<int> frc((size_t)nd, VS_OK);
+    {
+        std::vector<std::thread> th;
+        for (int i = 0; i < nd; ++i) th.emplace_back([&, i] { frc[(size_t)i] = vs::device_free_bytes(dev[(size_t)i], &free_b[(size_t)i]); });
+        for (auto &t : th) t.join();
+    }
+    for (int i = 0; i < nd; ++i)
+        if (frc[(size_t)i] != VS_OK) {
+            vs_set_last_error(("vs_mapper_create: device " + std::to_string(dev[(size_t)i]) + ": cannot read its free memory").c_str());
+            return frc[(size_t)i];
+        }
+    const int short_dev = vs::resident_plan_check(shape, text->n_words, free_b, need);
+    if (short_dev >= 0) {
+        vs_set_last_error(("vs_mapper_create: device " + std::to_string(dev[(size_t)short_dev]) + " needs " + std::to_string(need[(size_t)short_dev]) +
+                           " bytes for its " + std::to_string(n_shards / (size_t)nd) + " resident shard(s) but has " + std::to_string(free_b[(size_t)short_dev]) +
+                           " bytes free: spread the text over more devices").c_str());
+        return VS_ERR_NOMEM;
+    }
+    vs_mapper *m = new (std::nothrow) vs_mapper();
+    if (!m) return VS_ERR_NOMEM;
+    m->devices = dev;
+    m->bounds = b;
+    m->ctx.assign(n_shards, nullptr);
+    for (uint64_t x : need) m->planned_bytes += x;
+    std::string err;
+    const int rc = vs::for_each_shard(b, dev, &m->ctx, nullptr, err, [&](int, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *) {
+        return vs_text_upload(ctx, text, w0, n);
+    });
+    if (rc != VS_OK) {
+        vs_mapper_destroy(m);
+        vs_set_last_error(("vs_mapper_create: " + err).c_str());
+        return rc;
+    }
+    *out = m;
+    return VS_OK;
+}
+
+extern "C" int vs_mapper_map(vs_mapper *m, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam, int n_threads,
+                             vs_record **records, uint64_t *n_records, uint64_t *key16_collisions, vs_scan_stats *stats)
+{
+    if (records) *records = nullptr;
+    if (n_records) *n_records = 0;
+    if (!m || !records || !n_records || (n_guides && !guides)) { vs_set_last_error("vs_mapper_map: NULL argument"); return VS_ERR_ARG; }
+    if (k < 0 || k > VS_MAX_MISMATCHES) { vs_set_last_error("vs_mapper_map: mismatches must lie between 0 and 8"); return VS_ERR_ARG; }
+    if (extra_pam < -1 || extra_pam > 15) { vs_set_last_error("vs_mapper_map: extra_pam must be -1 or 4*x+y"); return VS_ERR_ARG; }
+    for (uint64_t i = 0; i < (uint64_t)n_guides * VS_GLEN; ++i)
+        if (guides[i] > 3) { vs_set_last_error("vs_mapper_map: guide codes must be 0..3"); return VS_ERR_ARG; }
+    bool idle = false;
+    if (!m->busy.compare_exchange_strong(idle, true)) { vs_set_last_error("vs_mapper_map: one call at a time on a mapper"); return VS_ERR_ARG; }
+    struct Release { std::atomic<bool> &b; ~Release() { b.store(false); } } release{m->busy};
+    std::vector<std::vector<vs_loc_hit>> lists(m->bounds.size() - 1);
+    std::string err;
+    int rc = vs::for_each_shard(m->bounds, m->devices, &m->ctx, stats, err, [&](int s, vs_ctx *ctx, uint64_t, uint64_t, vs_scan_stats *st) {
+        uint64_t cnt = 0;
+        return vs_scan_resolved(ctx, nullptr, 0, 0, guides, n_guides, k, extra_pam, nullptr, 0, &cnt, &vs::append_sink, &lists[(size_t)s], st);
+    });
+    if (rc != VS_OK) { vs_set_last_error(("vs_mapper_map: " + err).c_str()); return rc; }
+    return vs::merge_lists(lists, n_threads, records, n_records, key16_collisions);
+}
+
+extern "C" int vs_mapper_info(const vs_mapper *m, uint32_t *n_shards, uint64_t *device_bytes, uint64_t *planned_bytes)
+{
+    if (!m) { vs_set_last_error("vs_mapper_info: mapper is NULL"); return VS_ERR_ARG; }
+    uint32_t n = 0;
+    uint64_t bytes = 0;
+    for (const vs_ctx *c : m->ctx)
+        if (c) { ++n; bytes += vs::ctx_device_bytes(c); }
+    if (n_shards) *n_shards = n;
+    if (device_bytes) *device_bytes = bytes;
+    if (planned_bytes) *planned_bytes = m->planned_bytes;
+    return VS_OK;
+}
 
 extern "C" int vs_map_packed(const vs_text_view *text, const uint8_t *guides, uint32_t n_guides,
                              int k, int extra_pam, const int *devices, int n_devices,
@@ -921,17 +1075,7 @@ extern "C" int vs_map_records(const vs_text_view *text, const uint8_t *guides, u
     std::string err;
     int rc = vs::scan_text_sharded_resolved(*text, dev, guides, n_guides, k, extra_pam, lists, stats, err);
     if (rc != VS_OK) { vs_set_last_error(err.c_str()); return rc; }
-    std::vector<const vs_loc_hit *> ptr;
-    std::vector<uint64_t> cnt;
-    uint64_t total = 0;
-    for (auto &l : lists) { ptr.push_back(l.data()); cnt.push_back(l.size()); total += l.size(); }
-    if (total == 0) return VS_OK;
-    vs_record *o = (vs_record *)malloc(total * sizeof(vs_record));
-    if (!o) return VS_ERR_NOMEM;
-    rc = vs_merge_resolved(ptr.data(), cnt.data(), (int)ptr.size(), o, key16_collisions, n_threads);
-    if (rc != VS_OK) { free(o); return rc; }
-    *records = o; *n_records = total;
-    return VS_OK;
+    return vs::merge_lists(lists, n_threads, records, n_records, key16_collisions);
 }
 
 extern "C" int vs_shard_bounds(uint64_t n_words, int n_shards, uint64_t *out)

@@ -401,6 +401,69 @@ def map_records(text: PackedText, guides: np.ndarray, k: int, pam=None, devices=
     return rec, int(coll.value), st
 
 
+class Mapper:
+    """vs_mapper: map_records against a text kept resident in HBM.  The text is sharded over `devices` (default: device 0) as
+    map_records shards it and uploaded once; every shard keeps its candidate indexes, so later calls with the same PAM set only
+    score them (the bucketed index from the second call on, where the library's policy builds it).  Raises VarscotError with
+    VS_ERR_NOMEM when the shards and their indexes would not fit the devices' free memory."""
+
+    def __init__(self, text: PackedText, devices=None):
+        self._L = _lib.lib()
+        self._m = C.c_void_p()
+        dev = np.asarray(devices if devices else [0], dtype=np.int32)
+        v = text.view()
+        check(self._L.vs_mapper_create(C.byref(v), dev.ctypes.data, len(dev), C.byref(self._m)))
+        self.devices = [int(d) for d in dev]
+
+    def map(self, guides: np.ndarray, k: int, pam=None, threads: int = 1):
+        """Same as map_records(text, guides, k, pam, devices, threads): (records in emission order, key16_collisions, stats)."""
+        g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
+        rp, n, coll, st = C.c_void_p(), C.c_uint64(), C.c_uint64(), ScanStats()
+        check(self._L.vs_mapper_map(self._m, g.ctypes.data, g.shape[0], k, pam_code(pam) if not isinstance(pam, int) else pam, threads,
+                                    C.byref(rp), C.byref(n), C.byref(coll), C.byref(st)))
+        try:
+            rec = _copy_array(rp, n.value, REC_DT) if n.value else np.zeros(0, REC_DT)
+        finally:
+            self._L.vs_free(rp)
+        return rec, int(coll.value), st
+
+    def _info(self):
+        n, now, planned = C.c_uint32(), C.c_uint64(), C.c_uint64()
+        check(self._L.vs_mapper_info(self._m, C.byref(n), C.byref(now), C.byref(planned)))
+        return n.value, now.value, planned.value
+
+    @property
+    def n_shards(self) -> int:
+        return self._info()[0]
+
+    @property
+    def device_bytes(self) -> int:
+        """Device memory the mapper's contexts hold now."""
+        return self._info()[1]
+
+    @property
+    def planned_bytes(self) -> int:
+        """The create-time estimate of the device memory the resident shards need (all devices)."""
+        return self._info()[2]
+
+    def close(self):
+        if self._m:
+            self._L.vs_mapper_destroy(self._m)
+            self._m = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def shard_bounds(n_words: int, n_shards: int) -> np.ndarray:
     """vs_shard_bounds: word ranges owned by each of n_shards ranks / devices."""
     out = np.zeros(n_shards + 1, dtype=np.uint64)
