@@ -291,6 +291,76 @@ __device__ __forceinline__ uint32_t le_runtime(const uint32_t (&b)[5], int kp)
     else return kp == LO ? le_k<LO>(b) : le_runtime<LO + 1, HI>(b, kp);
 }
 
+// ---- the deal of a batch's segments to the CTA's warps ------------------------------------------------------------
+// A batch is scored by the CTA's warps between two barriers, so it lasts as long as its most loaded warp.  Its work is, per
+// class c = 0 .. min(K, VS_KEYLEN), one segment per 32 guides of the class and its tail in 4-guide segments (a 4-guide segment
+// walks 8 blocks per iteration, so a class costs 32 * n / 32 iterations however it is cut).  At 100 guides a bucket's classes
+// hold one 32-guide segment and a dozen or more 4-guide ones: dealt round robin by count, the warp that drew the 32-guide
+// segment also drew its share of the small ones while the three others waited at the barrier for a third of the batch.
+// The segments are therefore dealt longest first, each to the warp with the least cost dealt so far (LPT list scheduling:
+// the most loaded warp carries at most 4/3 of the optimum).
+// Cost of one segment in issue slots: set-up (perm and pattern loads, slot addresses) plus, per iteration, the walk's
+// stage-A loads, its carry-save adder tree (2 LOP3 per adder, pa - popc(pa) adders), threshold, vote and half an address
+// update per slot.  Only the ratios matter.
+constexpr uint32_t BK_SEG_SETUP = 60;
+__host__ __device__ inline uint32_t bk_segment_cost(int kp, uint32_t iters)
+{
+    const uint32_t pa = (uint32_t)bk_walk_slots(kp);
+#if defined(__CUDA_ARCH__) && !defined(VS_HOST_UNIT_TEST)
+    const uint32_t adders = pa - (uint32_t)__popc(pa);
+#else
+    const uint32_t adders = pa - (uint32_t)__builtin_popcount(pa);
+#endif
+    return BK_SEG_SETUP + iters * ((3u * pa) / 2u + 2u * adders + 4u);
+}
+// bk_deal: the deal of the segments of a bucket (class starts cls[0 .. BK_CLS)) to `warps` (<= SC_WARPS) warps, as RUNS: calls
+// emit(v, at, nseg, c, L, last) once per run — nseg consecutive segments of 2^L guide lanes (L = 5: 32 guides, L = 2: 4 guides)
+// of class c dealt to warp v, the first at perm entry `at`, the next 2^L entries further each, every one full but the last,
+// which holds `last` guides.  Order: the 32-guide segments by class, then the 4-guide ones by class (c ascending = stage-A
+// slots descending, so the cost never increases); ties go to the lowest warp.  The segments of one (class, shape) cost the
+// same, so what the greedy decides for them is how many each warp gets: a warp takes a contiguous run of them, and a warp
+// holds at most BK_RUNS runs.  It depends on the bucket only: k_score_bucketed computes it when its batches enter a new
+// bucket (about 47 batches per bucket at 3.5 Gbases) and rotates the warps per batch.
+constexpr int BK_RUNS = 2 * (VS_KEYLEN + 1);
+template <int K, class F>
+__host__ __device__ __forceinline__ void bk_deal(const uint32_t *cls, uint32_t warps, F &&emit)
+{
+    constexpr uint32_t CMAX = (uint32_t)(K < VS_KEYLEN ? K : VS_KEYLEN);   // a guide with c > K cannot hit in this bucket
+    uint32_t load[SC_WARPS];                                               // cost dealt so far per warp
+#pragma unroll
+    for (int v = 0; v < SC_WARPS; ++v) load[v] = 0u;
+#pragma unroll 1
+    for (uint32_t pass = 0; pass < 2u; ++pass) {
+#pragma unroll 1
+        for (uint32_t c = 0; c <= CMAX; ++c) {
+            const uint32_t c0 = cls[c], n = cls[c + 1] - c0, nfull = n & ~31u;
+            const uint32_t L = pass ? 2u : 5u, base = pass ? nfull : 0u, units = pass ? (n - nfull + 3u) >> 2 : nfull >> 5;
+            const uint32_t cost = bk_segment_cost(K - (int)c, pass ? 4u : 32u);
+            uint32_t cnt[SC_WARPS];
+#pragma unroll
+            for (int v = 0; v < SC_WARPS; ++v) cnt[v] = 0u;
+#pragma unroll 1
+            for (uint32_t u = 0; u < units; ++u) {
+                uint32_t best = 0u, least = load[0];
+#pragma unroll
+                for (uint32_t v = 1; v < (uint32_t)SC_WARPS; ++v)
+                    if (v < warps && load[v] < least) { best = v; least = load[v]; }
+#pragma unroll
+                for (uint32_t v = 0; v < (uint32_t)SC_WARPS; ++v)
+                    if (v == best) { load[v] += cost; ++cnt[v]; }
+            }
+            uint32_t i = base;
+#pragma unroll
+            for (uint32_t v = 0; v < (uint32_t)SC_WARPS; ++v)
+                if (cnt[v]) {
+                    const uint32_t end = i + (cnt[v] << L);
+                    emit(v, c0 + i, cnt[v], c, L, min(1u << L, n - (end - (1u << L))));
+                    i = end;
+                }
+        }
+    }
+}
+
 struct BkScoreArgs {
     const uint32_t *planes[2];  // bucketed store per strand
     const uint32_t *pos[2];     // bucketed positions per strand
@@ -370,6 +440,9 @@ k_score_bucketed(BkScoreArgs a)
     if (bat0 < bat1) stage(bat0);
     const uint32_t warps = blockDim.x >> 5;
     int bucket = -1, bucket_strand = -1;
+    __shared__ uint2 runs_s[SC_WARPS][SC_WARPS][BK_RUNS];   // per warp: the current bucket's deal, BK_RUNS runs per dealt warp
+    __shared__ uint32_t nrun_s[SC_WARPS][SC_WARPS];
+    int deal_bucket = -1, deal_strand = -1;
     for (unsigned long long bat = bat0; bat < bat1; ++bat) {
     const uint32_t strand = bat >= nbat_f;
     const unsigned long long blk0 = (bat - (strand ? nbat_f : 0ull)) * SC_NB;
@@ -383,6 +456,22 @@ k_score_bucketed(BkScoreArgs a)
     asm volatile("cp.async.wait_group 0;" ::: "memory");
 #endif
     __syncthreads();
+    if (deal_bucket != bucket || deal_strand != (int)strand) {
+        // the bucket's deal, computed by every lane and kept by its warp in shared memory (each warp writes and reads only its
+        // own copy; its lanes write the same values): recomputed when the batches enter a new bucket
+        uint32_t nr[SC_WARPS];
+#pragma unroll
+        for (int u = 0; u < SC_WARPS; ++u) nr[u] = 0u;
+        bk_deal<K>(a.cls + ((size_t)strand * BK_N + bucket) * BK_CLS, warps,
+                   [&](uint32_t v, uint32_t at, uint32_t nseg, uint32_t c, uint32_t L, uint32_t last) {
+#pragma unroll
+                       for (uint32_t u = 0; u < (uint32_t)SC_WARPS; ++u)
+                           if (u == v) runs_s[wid][u][nr[u]++] = uint2{at, nseg | (c << 16) | (L << 20) | (last << 24)};
+                   });
+#pragma unroll
+        for (int u = 0; u < SC_WARPS; ++u) nrun_s[wid][u] = nr[u];
+        deal_bucket = bucket; deal_strand = (int)strand;
+    }
     {
         const uint32_t b = (uint32_t)lane;
         const uint32_t inv = ~raw_s[BLK_VALID * SC_NB + b];
@@ -398,7 +487,6 @@ k_score_bucketed(BkScoreArgs a)
     const uint16_t *pat0 = a.pat + ((size_t)strand * a.pat_guides + a.guide_base) * PAT_STRIDE;
     const uint32_t *posb = (strand ? a.pos[1] : a.pos[0]) + blk0 * 32;
     const uint16_t *perm = a.perm + ((size_t)strand * BK_N + bucket) * a.n_guides;
-    const uint32_t *cls = a.cls + ((size_t)strand * BK_N + bucket) * BK_CLS;
 
     // The walk of one segment, stage A only: PA slots per iteration, (32 >> L) blocks per iteration.  Iterations in which some
     // lane is still within budget are noted in the returned mask and rescanned by bk_cold afterwards.  One copy of this code
@@ -459,19 +547,16 @@ k_score_bucketed(BkScoreArgs a)
         if (pend) bk_cold<K>(smb, step * ROW, pend, step, sub, po, kp, c, (int)strand, real, lastm_s, posb,
                              ((a.guide_base + g) << 8) | (strand << 7), a.hits, a.n_hits, a.hit_cap);
     };
-    // the segments of the batch — per class the full 32-guide segments, then its tail in 4-guide segments (a 4-guide segment
-    // walks 8 blocks per iteration, so a class costs 32 * n / 32 iterations however it is cut) — are dealt to the warps
-    // round robin; the deal starts at a different warp for every batch and CTA.  Classes c = 0 .. min(K, VS_KEYLEN): a
-    // guide with c > K cannot hit in this bucket.
-    uint32_t turn = (uint32_t)(bat + blockIdx.x) % warps;
-    for (uint32_t c = 0; c <= (uint32_t)(K < VS_KEYLEN ? K : VS_KEYLEN); ++c) {
-        const uint32_t c0 = cls[c], n = cls[c + 1] - c0;
-        for (uint32_t i = 0; i < n; ) {
-            const bool full = i + 32u <= n;
-            if (turn == (uint32_t)wid) segment(c0 + i, full ? 32u : min(4u, n - i), c, full ? 5u : 2u);
-            i += full ? 32u : 4u;
-            turn = turn + 1u == warps ? 0u : turn + 1u;
-        }
+    // the segments of the batch: the bucket's deal (bk_deal), its warps rotated by one for every batch and CTA so that no warp
+    // (and SM sub-partition) keeps the heavy share
+    const uint32_t v = (uint32_t)(wid + bat + blockIdx.x) % warps;
+    const uint32_t nrun = nrun_s[wid][v];
+#pragma unroll 1
+    for (uint32_t r = 0; r < nrun; ++r) {
+        const uint2 e = runs_s[wid][v][r];
+        const uint32_t nseg = e.y & 0xFFFFu, c = (e.y >> 16) & 0xFu, L = (e.y >> 20) & 0xFu, last = e.y >> 24;
+#pragma unroll 1
+        for (uint32_t j = 0; j < nseg; ++j) segment(e.x + (j << L), j + 1u < nseg ? 1u << L : last, c, L);
     }
     }
 }
