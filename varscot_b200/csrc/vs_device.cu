@@ -20,9 +20,41 @@ static thread_local std::string g_last_error;
 
 constexpr uint64_t DEFAULT_CHUNK_WORDS = 8ull << 20;      // 256 Mi bases per pipeline chunk
 
+// A grow-only buffer of a context: device memory, or pinned host memory when Pinned.  grow() is its only allocation and the
+// destructor frees it; a device buffer counts its bytes in its context's device_bytes while it holds them (ctx_device_bytes).
+template <typename T, bool Pinned = false>
+struct Buf {
+    T *p = nullptr;
+    uint64_t cap = 0;                    // elements
+    uint64_t *held = nullptr;            // device_bytes of the context that allocated it
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    ~Buf() { release(); }
+    operator T *() const { return p; }
+    int grow(vs_ctx *ctx, uint64_t n);
+    void release()
+    {
+        if (!p) return;
+        if (Pinned) cudaFreeHost(p);
+        else { cudaFree(p); *held -= cap * sizeof(T); }
+        p = nullptr; cap = 0;
+    }
+};
+template <typename T> using PinnedBuf = Buf<T, true>;
+
+// Buffers that are only used together: after one of them failed to grow, none of them holds memory.
+template <typename... B>
+static int release_all(B &...b)
+{
+    (b.release(), ...);
+    return VS_ERR_CUDA;
+}
+
 struct vs_ctx {
     int device = -1;
     int n_sm = 148;
+    uint64_t device_bytes = 0;           // sum of the capacities of the device buffers below (kept by Buf)
     cudaStream_t stream = nullptr;       // extraction + scoring + hit resolution
     cudaStream_t copy = nullptr;         // H2D of the next chunk (copies only, so that the copy engine never waits for a kernel)
     cudaStream_t prep = nullptr;         // small kernels that turn the uploaded mask source of a chunk into its window masks
@@ -32,29 +64,27 @@ struct vs_ctx {
     uint64_t chunk_words = DEFAULT_CHUNK_WORDS;
     // resident text shard: device word 0 = global word first_word; every position the device stores or emits (candidate
     // store, bucketed store, hits, contig starts) is global - pos_origin (see pos_origin_of)
-    vs_bases *d_bases = nullptr;
-    vs_masks *d_masks = nullptr;
-    uint64_t words_cap = 0, n_words = 0, first_word = 0, pos_origin = 0;
-    vs_mask_entry *d_sparse = nullptr;
-    uint64_t sparse_cap = 0;
+    Buf<vs_bases> d_bases;
+    Buf<vs_masks> d_masks;
+    uint64_t n_words = 0, first_word = 0, pos_origin = 0;
+    Buf<vs_mask_entry> d_sparse;
     // compact mask source path: the N and contig-end planes of the shard (+ halo word) and a staging area for their runs
-    uint32_t *d_nm = nullptr, *d_em = nullptr;
-    uint8_t *d_emcode = nullptr, *d_dense = nullptr;     // code bytes of the shard's contig-end plane; coded-block flags of the whole text
-    uint64_t planes_cap = 0, dense_cap = 0;
-    vs_plane_run *d_runs = nullptr;
-    uint64_t runs_cap = 0;
+    Buf<uint32_t> d_nm, d_em;
+    Buf<uint8_t> d_emcode, d_dense;      // code bytes of the shard's contig-end plane; coded-block flags of the whole text
+    Buf<vs_plane_run> d_runs;
     // contig starts of the shard (device-side hit resolution): derived from d_em, or uploaded
-    uint32_t *d_cstart = nullptr, *d_tilecnt = nullptr, *d_cs_total = nullptr, *h_cs_total = nullptr;
-    uint64_t cstart_cap = 0, tilecnt_cap = 0;
+    Buf<uint32_t> d_cstart, d_tilecnt, d_cs_total;
+    PinnedBuf<uint32_t> h_cs_total;
     uint32_t n_cstart = 0, first_contig = 0;
     bool cstart_valid = false;
     // counters (u64): [0..3] running candidates fwd / rev, block claims fwd / rev; [4 + 4 c ..] block range of chunk c
     // {lo fwd, lo rev, hi fwd, hi rev}; then the whole-store range [4]; then the hit counter
-    unsigned long long *d_cnt = nullptr, *h_cnt = nullptr;
-    uint64_t cnt_chunks = 0;
-    // candidate store of the whole shard, per strand (the resident index)
-    uint32_t *d_planes[2] = {nullptr, nullptr}, *d_pos[2] = {nullptr, nullptr};
-    uint64_t blocks_cap = 0;
+    Buf<unsigned long long> d_cnt;
+    PinnedBuf<unsigned long long> h_cnt;
+    uint64_t cnt_chunks = 0;             // the chunks d_cnt / h_cnt have room for: set once both have grown
+    // candidate store of the whole shard, per strand (the resident index): blocks of BLK_WORDS plane words and 32 positions
+    Buf<uint32_t> d_planes[2], d_pos[2];
+    uint64_t blocks_cap() const { return d_pos[0].cap / 32; }      // the four grow together (ensure_blocks)
     bool idx_valid = false;
     int idx_pam = -2;
     uint64_t idx_blocks[2] = {0, 0}, idx_cand[2] = {0, 0};
@@ -65,25 +95,25 @@ struct vs_ctx {
     // bucketed index (vs_bucket.cuh): the candidates regrouped by PAM kind + the VS_KEYLEN - 2 = 6 bases next to the PAM
     int bucket_mode = 1;                 // VS_OPT_BUCKET_INDEX: 0 never, 1 when a resident index is scanned again and it pays (guide count, shard size), 2 always
     bool bk_valid = false;
-    uint32_t *d_bk_planes[2] = {nullptr, nullptr}, *d_bk_pos[2] = {nullptr, nullptr};
-    uint64_t bk_cap[2] = {0, 0}, bk_blocks[2] = {0, 0};
-    unsigned long long *d_bk_ctl = nullptr, *h_bk_ctl = nullptr;     // hist [2][BK_N], cursor [2][BK_N], start [2][BK_N + 1]
-    uint16_t *d_perm = nullptr, *d_gkey = nullptr, *h_gkey = nullptr;
-    uint32_t *d_cls = nullptr;
-    uint64_t perm_cap = 0, gkey_cap = 0;
+    Buf<uint32_t> d_bk_planes[2], d_bk_pos[2];
+    uint64_t bk_blocks[2] = {0, 0};
+    Buf<unsigned long long> d_bk_ctl;    // hist [2][BK_N], cursor [2][BK_N], start [2][BK_N + 1]
+    PinnedBuf<unsigned long long> h_bk_ctl;
+    Buf<uint16_t> d_perm, d_gkey;
+    PinnedBuf<uint16_t> h_gkey;
+    Buf<uint32_t> d_cls;
     float bk_build_ms = 0.f;
     // pattern table [2][n_guides][PAT_STRIDE] of uint16
-    uint16_t *d_pat = nullptr, *h_pat = nullptr;
-    uint64_t pat_cap = 0;
+    Buf<uint16_t> d_pat;
+    PinnedBuf<uint16_t> h_pat;
     // hits
-    vs_hit *d_hits = nullptr;
-    uint64_t hits_cap = 0, last_n_hits = 0;
+    Buf<vs_hit> d_hits;
+    uint64_t last_n_hits = 0;
     // resolution: sort keys / payloads (double buffers of the radix sort), packed records, sort scratch, pinned staging
-    unsigned long long *d_keys[2] = {nullptr, nullptr}, *d_vals[2] = {nullptr, nullptr};
-    vs_loc_hit *d_loc = nullptr, *h_stage = nullptr;
-    uint64_t loc_cap = 0, stage_cap = 0;
-    void *d_sort_tmp = nullptr;
-    size_t sort_tmp_bytes = 0;
+    Buf<unsigned long long> d_keys[2], d_vals[2];
+    Buf<vs_loc_hit> d_loc;
+    PinnedBuf<vs_loc_hit> h_stage;
+    Buf<uint8_t> d_sort_tmp;
     std::string err;
 };
 
@@ -100,6 +130,27 @@ static int fail(vs_ctx *c, int code, const std::string &msg)
         if (e_ != cudaSuccess)                                                                     \
             return fail(ctx, VS_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));     \
     } while (0)
+
+template <typename T, bool Pinned>
+int Buf<T, Pinned>::grow(vs_ctx *ctx, uint64_t n)
+{
+    if (n <= cap) return VS_OK;
+    if (p) {
+        // any stream of the context may still use the old allocation (the copy and preparation streams fill the text, masks
+        // and planes that the scan stream reads): drain all three before it goes
+        for (cudaStream_t s : {ctx->stream, ctx->copy, ctx->prep}) CK(cudaStreamSynchronize(s));
+        release();
+    }
+    const size_t bytes = n * sizeof(T);
+    const cudaError_t e = Pinned ? cudaMallocHost(&p, bytes) : cudaMalloc(&p, bytes);
+    if (e != cudaSuccess) {
+        p = nullptr;
+        return fail(ctx, VS_ERR_CUDA, std::string(Pinned ? "cudaMallocHost(" : "cudaMalloc(") + std::to_string(bytes) + " bytes): " + cudaGetErrorString(e));
+    }
+    cap = n;
+    if (!Pinned) { held = &ctx->device_bytes; *held += bytes; }
+    return VS_OK;
+}
 
 extern "C" const char *vs_last_error(const vs_ctx *ctx)
 {
@@ -155,10 +206,9 @@ extern "C" int vs_ctx_create(int device, vs_ctx **out)
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_zeroed, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_starts, cudaEventDisableTiming);
     for (int i = 0; i < 8 && e == cudaSuccess; ++i) e = cudaEventCreate(&ctx->ev[i]);
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_cs_total, sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMallocHost(&ctx->h_cs_total, sizeof(uint32_t));
-    if (e != cudaSuccess) {
-        std::string m = std::string("vs_ctx_create: ") + cudaGetErrorString(e);
+    if (e != cudaSuccess) fail(ctx, VS_ERR_CUDA, cudaGetErrorString(e));
+    if (e != cudaSuccess || ctx->d_cs_total.grow(ctx, 1) != VS_OK || ctx->h_cs_total.grow(ctx, 1) != VS_OK) {
+        std::string m = "vs_ctx_create: " + ctx->err;
         vs_ctx_destroy(ctx);
         return fail(nullptr, VS_ERR_CUDA, m);
     }
@@ -170,24 +220,10 @@ extern "C" void vs_ctx_destroy(vs_ctx *ctx)
 {
     if (!ctx) return;
     if (ctx->device >= 0) cudaSetDevice(ctx->device);
+    // with the streams idle no work refers to a buffer; the buffers free themselves when ctx is deleted
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     if (ctx->copy) cudaStreamSynchronize(ctx->copy);
     if (ctx->prep) cudaStreamSynchronize(ctx->prep);
-    cudaFree(ctx->d_bases); cudaFree(ctx->d_masks); cudaFree(ctx->d_sparse);
-    cudaFree(ctx->d_nm); cudaFree(ctx->d_em); cudaFree(ctx->d_runs); cudaFree(ctx->d_emcode); cudaFree(ctx->d_dense);
-    cudaFree(ctx->d_cstart); cudaFree(ctx->d_tilecnt); cudaFree(ctx->d_cs_total);
-    if (ctx->h_cs_total) cudaFreeHost(ctx->h_cs_total);
-    cudaFree(ctx->d_cnt);
-    if (ctx->h_cnt) cudaFreeHost(ctx->h_cnt);
-    for (int s = 0; s < 2; ++s) { cudaFree(ctx->d_planes[s]); cudaFree(ctx->d_pos[s]); cudaFree(ctx->d_keys[s]); cudaFree(ctx->d_vals[s]); }
-    cudaFree(ctx->d_pat);
-    if (ctx->h_pat) cudaFreeHost(ctx->h_pat);
-    cudaFree(ctx->d_hits); cudaFree(ctx->d_loc); cudaFree(ctx->d_sort_tmp);
-    for (int s = 0; s < 2; ++s) { cudaFree(ctx->d_bk_planes[s]); cudaFree(ctx->d_bk_pos[s]); }
-    cudaFree(ctx->d_bk_ctl); cudaFree(ctx->d_perm); cudaFree(ctx->d_gkey); cudaFree(ctx->d_cls);
-    if (ctx->h_bk_ctl) cudaFreeHost(ctx->h_bk_ctl);
-    if (ctx->h_gkey) cudaFreeHost(ctx->h_gkey);
-    if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
     for (int i = 0; i < 8; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -221,20 +257,7 @@ extern "C" int vs_index_drop(vs_ctx *ctx)
 // ---- device memory accounting (vs_mapper) -----------------------------------------------------------------------------
 constexpr uint64_t BLOCK_BYTES = BLK_WORDS * 4 + 32 * 4;            // one block of 32 candidates: planes + positions
 
-uint64_t vs::ctx_device_bytes(const vs_ctx *ctx)
-{
-    if (!ctx) return 0;
-    uint64_t b = ctx->words_cap * (sizeof(vs_bases) + sizeof(vs_masks)) + ctx->sparse_cap * sizeof(vs_mask_entry);
-    b += ctx->planes_cap * (2 * sizeof(uint32_t) + 1) + ctx->dense_cap + ctx->runs_cap * sizeof(vs_plane_run);
-    b += (ctx->cstart_cap + ctx->tilecnt_cap + 1) * sizeof(uint32_t);
-    if (ctx->d_cnt) b += (4 + 4 * (ctx->cnt_chunks + 1) + 4 + 4) * sizeof(unsigned long long);
-    b += 2 * ctx->blocks_cap * BLOCK_BYTES + (ctx->bk_cap[0] + ctx->bk_cap[1]) * BLOCK_BYTES;
-    if (ctx->d_bk_ctl) b += (2 * BK_N + 2 * BK_N + 2 * (BK_N + 1)) * sizeof(unsigned long long);
-    if (ctx->d_cls) b += 2ull * BK_N * BK_CLS * sizeof(uint32_t);
-    b += (ctx->perm_cap + ctx->gkey_cap + ctx->pat_cap) * sizeof(uint16_t);
-    b += ctx->hits_cap * sizeof(vs_hit) + ctx->loc_cap * (4 * 8 + sizeof(vs_loc_hit)) + ctx->sort_tmp_bytes;
-    return b;
-}
+uint64_t vs::ctx_device_bytes(const vs_ctx *ctx) { return ctx ? ctx->device_bytes : 0; }
 
 // Candidate store of a shard, blocks per strand: the expected n_pam / 16 candidates per strand and base, + 15 %, + one partial
 // block per extraction tile and per chunk (what scan_engine allocates before the first extraction)
@@ -394,20 +417,6 @@ static std::vector<uint64_t> chunk_plan(uint64_t n_words, uint64_t chunk_words, 
 }
 
 // ---- text residency ------------------------------------------------------------------------------
-static int ensure_text_buffers(vs_ctx *ctx, uint64_t n_words)
-{
-    if (n_words + 1 > ctx->words_cap) {
-        CK(cudaStreamSynchronize(ctx->stream));
-        CK(cudaStreamSynchronize(ctx->copy));
-        cudaFree(ctx->d_bases); cudaFree(ctx->d_masks);
-        ctx->d_bases = nullptr; ctx->d_masks = nullptr; ctx->words_cap = 0;
-        CK(cudaMalloc(&ctx->d_bases, (n_words + 1) * sizeof(vs_bases)));
-        CK(cudaMalloc(&ctx->d_masks, (n_words + 1) * sizeof(vs_masks)));
-        ctx->words_cap = n_words + 1;
-    }
-    return VS_OK;
-}
-
 static inline bool has_mask_source(const vs_text_view *t) { return t->em_code && t->em_dense; }
 
 // runs of a sorted run list that overlap the word range [lo, hi): index range [first, last)
@@ -464,7 +473,7 @@ static int enqueue_chunk_copy(vs_ctx *ctx, const vs_text_view *t, uint64_t first
         auto stage = [&](const vs_plane_run *runs, uint64_t a, uint64_t b, vs_plane_run *&dst, uint64_t &cnt) -> int {
             cnt = b > a ? b - a : 0;
             if (!cnt) return VS_OK;
-            if (staged + cnt > ctx->runs_cap) return fail(ctx, VS_ERR_CUDA, "run staging area too small");
+            if (staged + cnt > ctx->d_runs.cap) return fail(ctx, VS_ERR_CUDA, "run staging area too small");
             dst = ctx->d_runs + staged;
             CK(cudaMemcpyAsync(dst, runs + a, cnt * sizeof(vs_plane_run), cudaMemcpyHostToDevice, cs));
             staged += cnt;
@@ -529,7 +538,7 @@ static int enqueue_chunk_copy(vs_ctx *ctx, const vs_text_view *t, uint64_t first
         const vs_mask_entry *sb = t->sparse, *se = t->sparse + t->n_sparse;
         auto lb = [&](uint64_t w) { return (uint64_t)(std::lower_bound(sb, se, w, [](const vs_mask_entry &x, uint64_t v) { return x.word < v; }) - sb); };
         e0 = lb(g0); e1 = lb(g0 + n);
-        sparse = (e1 - e0) * sizeof(vs_mask_entry) < n * sizeof(vs_masks) * 3 / 4 && staged + (e1 - e0) <= ctx->sparse_cap;
+        sparse = (e1 - e0) * sizeof(vs_mask_entry) < n * sizeof(vs_masks) * 3 / 4 && staged + (e1 - e0) <= ctx->d_sparse.cap;
     }
     if (sparse) {
         CK(cudaMemsetAsync(ctx->d_masks + c0, 0, n * sizeof(vs_masks), cs));
@@ -553,47 +562,20 @@ static int enqueue_chunk_copy(vs_ctx *ctx, const vs_text_view *t, uint64_t first
 static int ensure_sparse_staging(vs_ctx *ctx, const vs_text_view *t, uint64_t first_word, uint64_t n_words)
 {
     if (has_mask_source(t)) {
-        if (n_words + 1 > ctx->planes_cap) {
-            CK(cudaStreamSynchronize(ctx->copy));
-            cudaFree(ctx->d_nm); cudaFree(ctx->d_em); cudaFree(ctx->d_emcode);
-            ctx->d_nm = ctx->d_em = nullptr; ctx->d_emcode = nullptr; ctx->planes_cap = 0;
-            CK(cudaMalloc(&ctx->d_nm, (n_words + 1) * sizeof(uint32_t)));
-            CK(cudaMalloc(&ctx->d_em, (n_words + 1) * sizeof(uint32_t)));
-            CK(cudaMalloc(&ctx->d_emcode, n_words + 1));
-            ctx->planes_cap = n_words + 1;
-        }
-        const uint64_t n_blocks = (t->n_words + VS_EM_BLOCK) / VS_EM_BLOCK;
-        if (n_blocks > ctx->dense_cap) {
-            CK(cudaStreamSynchronize(ctx->copy));
-            CK(cudaStreamSynchronize(ctx->prep));
-            cudaFree(ctx->d_dense); ctx->d_dense = nullptr; ctx->dense_cap = 0;
-            CK(cudaMalloc(&ctx->d_dense, n_blocks));
-            ctx->dense_cap = n_blocks;
-        }
+        if (ctx->d_nm.grow(ctx, n_words + 1) || ctx->d_em.grow(ctx, n_words + 1) || ctx->d_emcode.grow(ctx, n_words + 1))
+            return release_all(ctx->d_nm, ctx->d_em, ctx->d_emcode);
+        int r;
+        if ((r = ctx->d_dense.grow(ctx, (t->n_words + VS_EM_BLOCK) / VS_EM_BLOCK)) != VS_OK) return r;
         uint64_t a0, a1, b0, b1;
         runs_in_range(t->nm_runs, t->n_nm_runs, first_word, first_word + n_words + 1, a0, a1);
         runs_in_range(t->em_runs, t->n_em_runs, first_word, first_word + n_words + 1, b0, b1);
         const uint64_t n_chunks = (n_words + ctx->chunk_words - 1) / ctx->chunk_words + 3;     // + the tapered tail of chunk_plan()
-        const uint64_t need = (a1 - a0) + (b1 - b0) + 4 * n_chunks + 16;
-        if (need > ctx->runs_cap) {
-            CK(cudaStreamSynchronize(ctx->copy));
-            cudaFree(ctx->d_runs); ctx->d_runs = nullptr; ctx->runs_cap = 0;
-            CK(cudaMalloc(&ctx->d_runs, need * sizeof(vs_plane_run)));
-            ctx->runs_cap = need;
-        }
-        return VS_OK;
+        return ctx->d_runs.grow(ctx, (a1 - a0) + (b1 - b0) + 4 * n_chunks + 16);
     }
     if (!t->sparse || t->n_sparse == 0) return VS_OK;
     const vs_mask_entry *sb = t->sparse, *se = t->sparse + t->n_sparse;
     auto lb = [&](uint64_t w) { return (uint64_t)(std::lower_bound(sb, se, w, [](const vs_mask_entry &x, uint64_t v) { return x.word < v; }) - sb); };
-    uint64_t need = lb(first_word + n_words) - lb(first_word);
-    if (need > ctx->sparse_cap) {
-        CK(cudaStreamSynchronize(ctx->copy));
-        cudaFree(ctx->d_sparse); ctx->d_sparse = nullptr; ctx->sparse_cap = 0;
-        CK(cudaMalloc(&ctx->d_sparse, need * sizeof(vs_mask_entry)));
-        ctx->sparse_cap = need;
-    }
-    return VS_OK;
+    return ctx->d_sparse.grow(ctx, lb(first_word + n_words) - lb(first_word));
 }
 
 // Start of an upload of a view with a compact mask source: zero both planes of the shard on the preparation stream
@@ -665,23 +647,18 @@ static int check_view(vs_ctx *ctx, const vs_text_view *t, uint64_t first_word, u
     return VS_OK;
 }
 
-static int ensure_starts_buffers(vs_ctx *ctx, const StartsPlan &p, uint64_t n_words)
+// Start of an upload of the shard [first_word, first_word + n_words) of t (vs_text_upload, or a scan that streams the text):
+// nothing is resident until it has completed; reserve the shard's text, staging and contig-start buffers.
+static int reserve_shard(vs_ctx *ctx, const vs_text_view *t, uint64_t first_word, uint64_t n_words, StartsPlan &sp)
 {
-    const uint64_t need = (uint64_t)(p.c_last - p.c_first) + 4;
-    if (need > ctx->cstart_cap) {
-        CK(cudaStreamSynchronize(ctx->stream)); CK(cudaStreamSynchronize(ctx->prep));
-        cudaFree(ctx->d_cstart); ctx->d_cstart = nullptr; ctx->cstart_cap = 0;
-        CK(cudaMalloc(&ctx->d_cstart, need * sizeof(uint32_t)));
-        ctx->cstart_cap = need;
-    }
-    const uint64_t tiles = (n_words + CS_TILE - 1) / CS_TILE + 1;
-    if (tiles > ctx->tilecnt_cap) {
-        CK(cudaStreamSynchronize(ctx->prep));
-        cudaFree(ctx->d_tilecnt); ctx->d_tilecnt = nullptr; ctx->tilecnt_cap = 0;
-        CK(cudaMalloc(&ctx->d_tilecnt, tiles * sizeof(uint32_t)));
-        ctx->tilecnt_cap = tiles;
-    }
-    return VS_OK;
+    ctx->n_words = 0; ctx->pos_origin = 0; ctx->idx_valid = false; ctx->bk_valid = false; ctx->cstart_valid = false;
+    if (ctx->d_bases.grow(ctx, n_words + 1) || ctx->d_masks.grow(ctx, n_words + 1)) return release_all(ctx->d_bases, ctx->d_masks);
+    int r;
+    if ((r = ensure_sparse_staging(ctx, t, first_word, n_words)) != VS_OK) return r;
+    sp = plan_contig_starts(t, first_word, n_words);
+    if (!sp.usable) return VS_OK;
+    if ((r = ctx->d_cstart.grow(ctx, (uint64_t)(sp.c_last - sp.c_first) + 4)) != VS_OK) return r;
+    return ctx->d_tilecnt.grow(ctx, (n_words + CS_TILE - 1) / CS_TILE + 1);
 }
 
 // enqueue the derivation from the contig-end plane on `st` (after the last chunk's planes are complete on that stream)
@@ -738,11 +715,8 @@ extern "C" int vs_text_upload(vs_ctx *ctx, const vs_text_view *t, uint64_t first
     if (r != VS_OK) return r;
     CK(cudaSetDevice(ctx->device));
     const uint64_t origin = pos_origin_of(t, first_word, n_words);
-    ctx->n_words = 0; ctx->pos_origin = 0; ctx->idx_valid = false; ctx->bk_valid = false; ctx->cstart_valid = false;      // nothing is resident until the upload has completed
-    if ((r = ensure_text_buffers(ctx, n_words)) != VS_OK) return r;
-    if ((r = ensure_sparse_staging(ctx, t, first_word, n_words)) != VS_OK) return r;
-    const StartsPlan sp = plan_contig_starts(t, first_word, n_words);
-    if (sp.usable && (r = ensure_starts_buffers(ctx, sp, n_words)) != VS_OK) return r;
+    StartsPlan sp;
+    if ((r = reserve_shard(ctx, t, first_word, n_words, sp)) != VS_OK) return r;
     uint64_t sparse_used = 0, bytes = 0;
     uint32_t launches = 0;
     cudaStream_t ready = ctx->copy;
@@ -782,11 +756,8 @@ static double hit_density(int k, int n_pam)
 static int build_bucket_index(vs_ctx *ctx, const PamParams &pp, uint32_t &launches)
 {
     cudaStream_t st = ctx->stream;
-    const size_t ctl_words = 2 * BK_N + 2 * BK_N + 2 * (BK_N + 1);
-    if (!ctx->d_bk_ctl) {
-        CK(cudaMalloc(&ctx->d_bk_ctl, ctl_words * sizeof(unsigned long long)));
-        CK(cudaMallocHost(&ctx->h_bk_ctl, 2 * (BK_N + 1) * sizeof(unsigned long long)));
-    }
+    if (ctx->d_bk_ctl.grow(ctx, 2 * BK_N + 2 * BK_N + 2 * (BK_N + 1)) || ctx->h_bk_ctl.grow(ctx, 2 * (BK_N + 1)))
+        return release_all(ctx->d_bk_ctl, ctx->h_bk_ctl);
     unsigned long long *d_hist = ctx->d_bk_ctl, *d_cursor = d_hist + 2 * BK_N, *d_start = d_cursor + 2 * BK_N;
     const unsigned long long *d_all = ctx->d_cnt + 4 + 4 * (ctx->cnt_chunks + 1);
     CK(cudaEventRecord(ctx->ev[7], st));
@@ -807,13 +778,10 @@ static int build_bucket_index(vs_ctx *ctx, const PamParams &pp, uint32_t &launch
     for (int s = 0; s < 2; ++s) {
         const uint64_t nb = ctx->h_bk_ctl[s * (BK_N + 1) + BK_N];
         ctx->bk_blocks[s] = nb;
-        if (nb > ctx->bk_cap[s]) {
-            cudaFree(ctx->d_bk_planes[s]); cudaFree(ctx->d_bk_pos[s]);
-            ctx->d_bk_planes[s] = ctx->d_bk_pos[s] = nullptr; ctx->bk_cap[s] = 0;
+        if (nb > ctx->d_bk_pos[s].cap / 32) {
             const uint64_t cap = nb + nb / 64 + SC_NB;
-            CK(cudaMalloc(&ctx->d_bk_planes[s], cap * BLK_WORDS * sizeof(uint32_t)));
-            CK(cudaMalloc(&ctx->d_bk_pos[s], cap * 32 * sizeof(uint32_t)));
-            ctx->bk_cap[s] = cap;
+            if (ctx->d_bk_planes[s].grow(ctx, cap * BLK_WORDS) || ctx->d_bk_pos[s].grow(ctx, cap * 32))
+                return release_all(ctx->d_bk_planes[s], ctx->d_bk_pos[s]);
         }
         if (nb) CK(cudaMemsetAsync(ctx->d_bk_pos[s], 0xFF, nb * 32 * sizeof(uint32_t), st));
     }
@@ -882,13 +850,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
     const uint64_t first_word = src ? q.first_word : ctx->first_word;
     const uint64_t origin = src ? pos_origin_of(src, first_word, n_words) : ctx->pos_origin;
     StartsPlan sp;
-    if (src) {
-        ctx->n_words = 0; ctx->pos_origin = 0; ctx->idx_valid = false; ctx->bk_valid = false; ctx->cstart_valid = false;      // nothing is resident until the pass has completed
-        if ((r = ensure_text_buffers(ctx, n_words)) != VS_OK) return r;
-        if ((r = ensure_sparse_staging(ctx, src, first_word, n_words)) != VS_OK) return r;
-        sp = plan_contig_starts(src, first_word, n_words);
-        if (sp.usable && (r = ensure_starts_buffers(ctx, sp, n_words)) != VS_OK) return r;
-    }
+    if (src && (r = reserve_shard(ctx, src, first_word, n_words, sp)) != VS_OK) return r;
     if (n_words == 0 || n_guides == 0) {
         if (src && n_words) { r = vs_text_upload(ctx, src, first_word, n_words); if (r != VS_OK) return r; }
         if (q.stats) *q.stats = S;
@@ -912,14 +874,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
 
     // pattern table [strand][guide][PAT_STRIDE] (uint16 plane offsets, see pat_slot), staged in pinned memory
     const uint64_t pat_entries = 2ull * n_guides * PAT_STRIDE;
-    if (pat_entries > ctx->pat_cap) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(ctx->d_pat); if (ctx->h_pat) cudaFreeHost(ctx->h_pat);
-        ctx->d_pat = ctx->h_pat = nullptr; ctx->pat_cap = 0;
-        CK(cudaMalloc(&ctx->d_pat, pat_entries * sizeof(uint16_t)));
-        CK(cudaMallocHost(&ctx->h_pat, pat_entries * sizeof(uint16_t)));
-        ctx->pat_cap = pat_entries;
-    }
+    if (ctx->d_pat.grow(ctx, pat_entries) || ctx->h_pat.grow(ctx, pat_entries)) return release_all(ctx->d_pat, ctx->h_pat);
     for (int s = 0; s < 2; ++s)
         for (uint32_t g = 0; g < n_guides; ++g) {
             uint16_t *dst = ctx->h_pat + ((size_t)s * n_guides + g) * PAT_STRIDE;
@@ -933,32 +888,22 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
         }
     // counters
     if (n_chunks > ctx->cnt_chunks) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(ctx->d_cnt); if (ctx->h_cnt) cudaFreeHost(ctx->h_cnt);
-        ctx->d_cnt = ctx->h_cnt = nullptr; ctx->cnt_chunks = 0;
-        uint64_t nc = n_chunks + 8;
-        CK(cudaMalloc(&ctx->d_cnt, (4 + 4 * (nc + 1) + 4 + 4) * sizeof(unsigned long long)));
-        CK(cudaMallocHost(&ctx->h_cnt, (4 + 4 * (nc + 1) + 4 + 4) * sizeof(unsigned long long)));
-        ctx->cnt_chunks = nc;
+        const uint64_t nc = n_chunks + 8, words = 4 + 4 * (nc + 1) + 4 + 4;
+        ctx->cnt_chunks = 0;
         ctx->idx_valid = false; ctx->bk_valid = false;       // the whole-store range lived in the old buffer
+        if (ctx->d_cnt.grow(ctx, words) || ctx->h_cnt.grow(ctx, words)) return release_all(ctx->d_cnt, ctx->h_cnt);
+        ctx->cnt_chunks = nc;
     }
     const uint64_t cnt_words = 4 + 4 * (ctx->cnt_chunks + 1) + 4 + 4;
     unsigned long long *d_rng = ctx->d_cnt + 4, *d_all = ctx->d_cnt + 4 + 4 * (ctx->cnt_chunks + 1), *d_hitcnt = d_all + 4;
     unsigned long long *h_rng = ctx->h_cnt + 4, *h_hitcnt = ctx->h_cnt + (d_hitcnt - ctx->d_cnt);
     // candidate store sized for the shard at the expected density (+15 %), regrown when it overflows
     auto ensure_blocks = [&](uint64_t need) -> int {
-        if (need <= ctx->blocks_cap) return VS_OK;
-        CK(cudaStreamSynchronize(st));
-        for (int s = 0; s < 2; ++s) {
-            cudaFree(ctx->d_planes[s]); cudaFree(ctx->d_pos[s]);
-            ctx->d_planes[s] = ctx->d_pos[s] = nullptr;
-        }
-        ctx->blocks_cap = 0; ctx->idx_valid = false; ctx->bk_valid = false;
-        for (int s = 0; s < 2; ++s) {
-            CK(cudaMalloc(&ctx->d_planes[s], need * BLK_WORDS * sizeof(uint32_t)));
-            CK(cudaMalloc(&ctx->d_pos[s], need * 32 * sizeof(uint32_t)));
-        }
-        ctx->blocks_cap = need;
+        if (need <= ctx->blocks_cap()) return VS_OK;
+        ctx->idx_valid = false; ctx->bk_valid = false;
+        for (int s = 0; s < 2; ++s)
+            if (ctx->d_planes[s].grow(ctx, need * BLK_WORDS) || ctx->d_pos[s].grow(ctx, need * 32))
+                return release_all(ctx->d_planes[0], ctx->d_pos[0], ctx->d_planes[1], ctx->d_pos[1]);
         return VS_OK;
     };
     const bool reuse = !src && ctx->idx_valid && ctx->idx_pam == q.extra_pam;
@@ -981,15 +926,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
     }
     if (use_bk) {
         // keys of the patterns and, per guide pass, the guides of every bucket sorted by their key mismatches
-        const uint64_t gk = 2ull * n_guides;
-        if (gk > ctx->gkey_cap) {
-            CK(cudaStreamSynchronize(st));
-            cudaFree(ctx->d_gkey); if (ctx->h_gkey) cudaFreeHost(ctx->h_gkey);
-            ctx->d_gkey = ctx->h_gkey = nullptr; ctx->gkey_cap = 0;
-            CK(cudaMalloc(&ctx->d_gkey, gk * sizeof(uint16_t)));
-            CK(cudaMallocHost(&ctx->h_gkey, gk * sizeof(uint16_t)));
-            ctx->gkey_cap = gk;
-        }
+        if (ctx->d_gkey.grow(ctx, 2ull * n_guides) || ctx->h_gkey.grow(ctx, 2ull * n_guides)) return release_all(ctx->d_gkey, ctx->h_gkey);
         for (int s = 0; s < 2; ++s)
             for (uint32_t g = 0; g < n_guides; ++g) {
                 uint8_t patc[VS_GLEN];
@@ -997,23 +934,15 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
                 for (int i = 0; i < VS_GLEN; ++i) patc[i] = s ? (uint8_t)(3 - gd[VS_GLEN - 1 - i]) : gd[i];
                 ctx->h_gkey[(size_t)s * n_guides + g] = (uint16_t)key_of_codes(s, patc);
             }
-        if (!ctx->d_cls) CK(cudaMalloc(&ctx->d_cls, 2ull * BK_N * BK_CLS * sizeof(uint32_t)));
+        if ((r = ctx->d_cls.grow(ctx, 2ull * BK_N * BK_CLS)) != VS_OK) return r;
     }
     // hit buffer and guide super-chunks
     const double per_guide = (double)n_words * 32.0 * hit_density(k, pp.n);
     uint64_t want_hits = ctx->hit_cap_opt ? ctx->hit_cap_opt
                                           : std::min<uint64_t>(64ull << 20, std::max<uint64_t>(4ull << 20, (uint64_t)(per_guide * n_guides * 1.5) + 65536));
-    auto ensure_hits = [&](uint64_t cap) -> int {
-        if (cap <= ctx->hits_cap) return VS_OK;
-        CK(cudaStreamSynchronize(st));
-        cudaFree(ctx->d_hits); ctx->d_hits = nullptr; ctx->hits_cap = 0;
-        CK(cudaMalloc(&ctx->d_hits, cap * sizeof(vs_hit)));
-        ctx->hits_cap = cap;
-        return VS_OK;
-    };
-    if ((r = ensure_hits(want_hits)) != VS_OK) return r;
+    if ((r = ctx->d_hits.grow(ctx, want_hits)) != VS_OK) return r;
     auto guides_per_pass = [&]() -> uint32_t {
-        const double fit = per_guide > 0 ? (double)ctx->hits_cap / (per_guide * 1.5) : 1e30;
+        const double fit = per_guide > 0 ? (double)ctx->d_hits.cap / (per_guide * 1.5) : 1e30;
         uint64_t g = fit >= (double)n_guides ? n_guides : (uint64_t)std::max(1.0, fit);
         if (g > 32768) g = 32768;                            // the sort key holds 15 bits of guide index per delivery (and k_guide_classes 16)
         if (g < n_guides && g > SC_THREADS) g = g / SC_THREADS * SC_THREADS;
@@ -1041,17 +970,17 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
         const uint64_t c0 = plan[c], c1 = plan[c + 1];
         const unsigned tiles = (unsigned)((c1 - c0 + tile_words - 1) / tile_words);
         k_extract<<<tiles, EX_THREADS, 0, st>>>(ctx->d_bases, ctx->d_masks, c0, c1, tile_words, first_word * 32 - origin, pp,
-                                                 ctx->d_planes[0], ctx->d_pos[0], ctx->d_planes[1], ctx->d_pos[1], ctx->blocks_cap, ctx->d_cnt);
-        k_extract_mark<<<1, 32, 0, st>>>(ctx->d_cnt, d_rng + 4ull * c, d_all, ctx->d_planes[0], ctx->d_planes[1], ctx->blocks_cap);
+                                                 ctx->d_planes[0], ctx->d_pos[0], ctx->d_planes[1], ctx->d_pos[1], ctx->blocks_cap(), ctx->d_cnt);
+        k_extract_mark<<<1, 32, 0, st>>>(ctx->d_cnt, d_rng + 4ull * c, d_all, ctx->d_planes[0], ctx->d_planes[1], ctx->blocks_cap());
         S.launches += 2;
     };
     auto launch_score = [&](const unsigned long long *rng, uint32_t g0, uint32_t ng) {
         ScoreArgs a;
         for (int s = 0; s < 2; ++s) { a.planes[s] = ctx->d_planes[s]; a.pos[s] = ctx->d_pos[s]; }
-        a.rng = rng; a.cap = ctx->blocks_cap;
+        a.rng = rng; a.cap = ctx->blocks_cap();
         a.n_guides = ng; a.guide_base = g0; a.pat_guides = n_guides; a.pat = ctx->d_pat;
         a.rot_shift = (uint32_t)rot_shift;
-        a.hits = ctx->d_hits; a.n_hits = d_hitcnt; a.hit_cap = ctx->hits_cap;
+        a.hits = ctx->d_hits; a.n_hits = d_hitcnt; a.hit_cap = ctx->d_hits.cap;
         dispatch_score(k, a, score_ctas, score_cta(ng), st);
         S.launches++; S.score_launches++;
     };
@@ -1075,13 +1004,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
                 // the index is resident: one launch over the whole store
                 CK(cudaEventRecord(ctx->ev[2], st));
                 if (use_bk) {
-                    const uint64_t need = 2ull * BK_N * ng;
-                    if (need > ctx->perm_cap) {
-                        CK(cudaStreamSynchronize(st));
-                        cudaFree(ctx->d_perm); ctx->d_perm = nullptr; ctx->perm_cap = 0;
-                        CK(cudaMalloc(&ctx->d_perm, need * sizeof(uint16_t)));
-                        ctx->perm_cap = need;
-                    }
+                    if ((r = ctx->d_perm.grow(ctx, 2ull * BK_N * ng)) != VS_OK) return r;
                     // the keys of this pass's guides, strand by strand ([2][ng])
                     for (int s = 0; s < 2; ++s)
                         CK(cudaMemcpyAsync(ctx->d_gkey + (size_t)s * ng, ctx->h_gkey + (size_t)s * n_guides + g0, (size_t)ng * sizeof(uint16_t), cudaMemcpyHostToDevice, st));
@@ -1092,7 +1015,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
                     b.start = ctx->d_bk_ctl + 4 * BK_N;
                     b.n_guides = ng; b.guide_base = g0; b.pat_guides = n_guides; b.pat = ctx->d_pat;
                     b.perm = ctx->d_perm; b.cls = ctx->d_cls;
-                    b.hits = ctx->d_hits; b.n_hits = d_hitcnt; b.hit_cap = ctx->hits_cap;
+                    b.hits = ctx->d_hits; b.n_hits = d_hitcnt; b.hit_cap = ctx->d_hits.cap;
                     dispatch_score_bk(k, b, score_ctas, SC_THREADS, st);
                     S.launches += 2; S.score_launches++;
                 } else {
@@ -1144,7 +1067,7 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
                     source = nullptr;
                 }
                 const uint64_t bf = ctx->h_cnt[2], br = ctx->h_cnt[3];
-                if (std::max(bf, br) > ctx->blocks_cap) {    // the store overflowed (k_score skipped everything): regrow, extract again
+                if (std::max(bf, br) > ctx->blocks_cap()) {    // the store overflowed (k_score skipped everything): regrow, extract again
                     uint64_t need = std::max(bf, br);
                     need = (need + need / 32 + 64ull * n_chunks + BLK_GROUP) / BLK_GROUP * BLK_GROUP;
                     if ((r = ensure_blocks(need)) != VS_OK) return r;
@@ -1169,11 +1092,11 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
                 S.score_ms += b;
             }
             found = *h_hitcnt;
-            if (found <= ctx->hits_cap) break;
+            if (found <= ctx->d_hits.cap) break;
             // device hit buffer too small: grow it (or halve the super-chunk once it is large) and repeat the pass over the index
             S.redo_chunks += n_chunks;
             if (found > (256ull << 20) && ng > 1) { ng = (ng + 1) / 2; continue; }
-            if ((r = ensure_hits(found + found / 8 + 1024)) != VS_OK) return r;
+            if ((r = ctx->d_hits.grow(ctx, found + found / 8 + 1024)) != VS_OK) return r;
         }
         S.guide_passes++;
         first_pass = false;
@@ -1185,38 +1108,27 @@ static int scan_engine(vs_ctx *ctx, const ScanReq &q)
             S.d2h_bytes += ncopy * sizeof(vs_hit);
             if (found > room) out_overflow = true;
         } else if (found) {
-            if (found > ctx->loc_cap) {
-                for (int s = 0; s < 2; ++s) { cudaFree(ctx->d_keys[s]); cudaFree(ctx->d_vals[s]); ctx->d_keys[s] = ctx->d_vals[s] = nullptr; }
-                cudaFree(ctx->d_loc); ctx->d_loc = nullptr; ctx->loc_cap = 0;
+            if (found > ctx->d_loc.cap) {
                 const uint64_t cap = std::max<uint64_t>(found + found / 8, 1u << 16);
-                for (int s = 0; s < 2; ++s) { CK(cudaMalloc(&ctx->d_keys[s], cap * 8)); CK(cudaMalloc(&ctx->d_vals[s], cap * 8)); }
-                CK(cudaMalloc(&ctx->d_loc, cap * sizeof(vs_loc_hit)));
-                ctx->loc_cap = cap;
+                if (ctx->d_keys[0].grow(ctx, cap) || ctx->d_keys[1].grow(ctx, cap) || ctx->d_vals[0].grow(ctx, cap) || ctx->d_vals[1].grow(ctx, cap) ||
+                    ctx->d_loc.grow(ctx, cap))
+                    return release_all(ctx->d_keys[0], ctx->d_keys[1], ctx->d_vals[0], ctx->d_vals[1], ctx->d_loc);
             }
             int guide_bits = 1;
             while ((1u << guide_bits) < ng) ++guide_bits;
             cub::DoubleBuffer<unsigned long long> dk(ctx->d_keys[0], ctx->d_keys[1]), dv(ctx->d_vals[0], ctx->d_vals[1]);
             size_t tmp = 0;
             CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, dk, dv, (unsigned long long)found, 0, 49 + guide_bits, st));
-            if (tmp > ctx->sort_tmp_bytes) {
-                cudaFree(ctx->d_sort_tmp); ctx->d_sort_tmp = nullptr; ctx->sort_tmp_bytes = 0;
-                CK(cudaMalloc(&ctx->d_sort_tmp, tmp + tmp / 4));
-                ctx->sort_tmp_bytes = tmp + tmp / 4;
-            }
+            if (tmp > ctx->d_sort_tmp.cap && (r = ctx->d_sort_tmp.grow(ctx, tmp + tmp / 4)) != VS_OK) return r;
             const unsigned gb = (unsigned)((found + 255) / 256);
             k_resolve_hits<<<gb, 256, 0, st>>>(ctx->d_hits, found, ctx->d_cstart, ctx->n_cstart, ctx->first_contig, g0, ctx->d_keys[0], ctx->d_vals[0]);
-            tmp = ctx->sort_tmp_bytes;
+            tmp = ctx->d_sort_tmp.cap;
             CK(cub::DeviceRadixSort::SortPairs(ctx->d_sort_tmp, tmp, dk, dv, (unsigned long long)found, 0, 49 + guide_bits, st));
             k_pack_loc_hits<<<gb, 256, 0, st>>>(dk.Current(), dv.Current(), found, ctx->d_loc);
             S.launches += 2 + 8;                              // + the radix sort's passes (CUB: histogram + one pass per 8 key bits)
             CK(cudaGetLastError());
             if (q.sink) {
-                if (found > ctx->stage_cap) {
-                    if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-                    ctx->h_stage = nullptr; ctx->stage_cap = 0;
-                    CK(cudaMallocHost(&ctx->h_stage, (found + found / 8) * sizeof(vs_loc_hit)));
-                    ctx->stage_cap = found + found / 8;
-                }
+                if (found > ctx->h_stage.cap && (r = ctx->h_stage.grow(ctx, found + found / 8)) != VS_OK) return r;
                 CK(cudaMemcpyAsync(ctx->h_stage, ctx->d_loc, found * sizeof(vs_loc_hit), cudaMemcpyDeviceToHost, st));
                 S.d2h_bytes += found * sizeof(vs_loc_hit);
             } else {
@@ -1322,8 +1234,9 @@ extern "C" int vs_measure_int_peaks(vs_ctx *ctx, double *lop3_per_s, double *lds
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, ctx->device));
     const int grid = prop.multiProcessorCount * 8, threads = 256, iters = 4096;
-    uint32_t *d_out = nullptr;
-    CK(cudaMalloc(&d_out, (size_t)grid * threads * sizeof(uint32_t)));
+    Buf<uint32_t> d_out;
+    int r;
+    if ((r = d_out.grow(ctx, (uint64_t)grid * threads)) != VS_OK) return r;
     cudaStream_t st = ctx->stream;
     float best_lop = 1e30f, best_lds = 1e30f;
     for (int rep = 0; rep < 5; ++rep) {
@@ -1342,7 +1255,6 @@ extern "C" int vs_measure_int_peaks(vs_ctx *ctx, double *lop3_per_s, double *lds
         if (rep && ms < best_lds) best_lds = ms;
     }
     CK(cudaGetLastError());
-    cudaFree(d_out);
     const double nthreads = (double)grid * threads;
     if (lop3_per_s) *lop3_per_s = nthreads * iters * 64.0 / (best_lop * 1e-3);
     if (lds_words_per_s) *lds_words_per_s = nthreads * iters * 8.0 / (best_lds * 1e-3);
