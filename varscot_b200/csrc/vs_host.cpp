@@ -1007,10 +1007,10 @@ extern "C" int vs_mapper_map(vs_mapper *m, const uint8_t *guides, uint32_t n_gui
     if (records) *records = nullptr;
     if (n_records) *n_records = 0;
     if (!m || !records || !n_records || (n_guides && !guides)) { vs_set_last_error("vs_mapper_map: NULL argument"); return VS_ERR_ARG; }
-    if (k < 0 || k > VS_MAX_MISMATCHES) { vs_set_last_error("vs_mapper_map: mismatches must lie between 0 and 8"); return VS_ERR_ARG; }
-    if (extra_pam < -1 || extra_pam > 15) { vs_set_last_error("vs_mapper_map: extra_pam must be -1 or 4*x+y"); return VS_ERR_ARG; }
-    for (uint64_t i = 0; i < (uint64_t)n_guides * VS_GLEN; ++i)
-        if (guides[i] > 3) { vs_set_last_error("vs_mapper_map: guide codes must be 0..3"); return VS_ERR_ARG; }
+    if (const char *why = vs::scan_arg_error(guides, n_guides, k, extra_pam)) {
+        vs_set_last_error((std::string("vs_mapper_map: ") + why).c_str());
+        return VS_ERR_ARG;
+    }
     bool idle = false;
     if (!m->busy.compare_exchange_strong(idle, true)) { vs_set_last_error("vs_mapper_map: one call at a time on a mapper"); return VS_ERR_ARG; }
     struct Release { std::atomic<bool> &b; ~Release() { b.store(false); } } release{m->busy};

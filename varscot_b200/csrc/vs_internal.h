@@ -12,6 +12,10 @@ void vs_warmup_device(int device);
 
 namespace vs {
 
+// Why the guides, mismatch count and extra PAM of a scan are rejected, or nullptr when they are valid.  Callers check them
+// before touching any device or resident state and prefix the reason with their own name.
+const char *scan_arg_error(const uint8_t *guides, uint32_t n_guides, int k, int extra_pam);
+
 // Scan a packed text on one or several devices (text sharded by word ranges as shard_plan, one host thread and one
 // context per device, no collective) and return all hits, unordered.  devices empty -> device 0.
 int scan_text_sharded(const vs_text_view &text, const std::vector<int> &devices,
