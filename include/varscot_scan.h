@@ -306,6 +306,38 @@ int  vs_mapper_create(const vs_text_view *text, const int *devices, int n_device
  * leaves the resident shards and indexes as they were; so does a call made while another one runs on the same mapper. */
 int  vs_mapper_map(vs_mapper *m, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam, int n_threads,
                    vs_record **records, uint64_t *n_records, uint64_t *key16_collisions, vs_scan_stats *stats);
+/* ---- streamed records ------------------------------------------------------------------------------------------
+ * The records of vs_mapper_map / vs_map_records delivered a range of whole guides at a time, in emission order, while the
+ * devices score the next range: host memory stays bounded by the delivery size instead of growing with the whole map.  The
+ * concatenated deliveries are, byte for byte, the records the one-shot call returns.
+ *   records_per_delivery  target records per delivery; 0 = 32 Mi.  A delivery holds whole guides (the flags are per guide
+ *                         and strand) and at most this many records, except a single guide denser than it, which comes alone.
+ *                         Ranges are sized from the expected hit density first, then from the hits per guide just scanned.
+ *   with_windows          also deliver each record's 23-base genome window, read on the device beside the sorted hit:
+ *                         bits 2 i .. 2 i + 1 = Dna code (A 0, C 1, G 2, T 3) of genome base pos + i of the record's contig,
+ *                         forward orientation.  vs_md_from_window turns it into the record's MD:Z without the host text.
+ *   sink                  called on the calling thread, one delivery at a time, guides ascending and contiguous from 0 to
+ *                         n_guides (a range without records is delivered too, with n = 0).  Record guide ids are absolute.
+ *                         The pointers are valid during the call only.  A non-zero return stops the call: no further sink
+ *                         call is made, the devices are drained, and the call returns VS_ERR_ARG ("the sink aborted").
+ * Host memory in flight: about 3 x records_per_delivery x (16 + 8 with_windows) bytes (the sorted lists of the range being
+ * delivered and of the range being scanned, and the merged delivery), plus every context's pinned staging of its largest
+ * super-chunk.  key16_collisions and stats are sums over the deliveries (times: device times summed over the ranges). */
+typedef int (*vs_record_sink)(void *user, const vs_record *records, const uint64_t *windows /* NULL unless asked */,
+                              uint64_t n, uint32_t guide_lo, uint32_t guide_hi);          /* non-zero aborts */
+/* The resident mapper's shards scan every range; the one-call-at-a-time rule of vs_mapper_map applies, and an abort leaves the
+ * resident shards and indexes as they were. */
+int vs_mapper_map_stream(vs_mapper *m, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam, int n_threads,
+                         uint64_t records_per_delivery, int with_windows, vs_record_sink sink, void *user,
+                         uint64_t *key16_collisions, vs_scan_stats *stats);
+/* Shards as vs_map_records.  With one shard per device every device keeps its context for the whole call: the first range
+ * streams the upload and extracts the candidate index, later ranges score the resident index.  With several shards per device
+ * (texts beyond 4 Gbases on few devices) every range uploads each shard again: that cost is paid only when the map needs more
+ * than one delivery. */
+int vs_map_records_stream(const vs_text_view *text, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
+                          const int *devices, int n_devices, int n_threads, uint64_t records_per_delivery, int with_windows,
+                          vs_record_sink sink, void *user, uint64_t *key16_collisions, vs_scan_stats *stats);
+
 /* shards held; bytes of device memory the mapper's contexts hold now, and the create-time estimate (all devices; an upper
  * bound for scans that keep up to 16 Mi hits per shard and pass, of up to 4096 guides) */
 int  vs_mapper_info(const vs_mapper *m, uint32_t *n_shards, uint64_t *device_bytes, uint64_t *planned_bytes);
@@ -315,6 +347,8 @@ void vs_mapper_destroy(vs_mapper *m);
 #define VS_MD_SAMTOOLS 1
 /* MD:Z value for the window at global position gpos against guide (codes) on the given strand. out >= 64 bytes. */
 int vs_md_string(const vs_bases *bases, uint64_t gpos, const uint8_t *guide, int strand, int md_style, char *out);
+/* MD:Z from a delivered window (vs_record_sink): the same string vs_md_string writes for that record. out >= 64 bytes. */
+int vs_md_from_window(uint64_t window, const uint8_t *guide, int strand, int md_style, char *out);
 /* one 13-column SAM line (R9) incl. '\n'; returns the length written (excluding NUL), or -1 if buflen is too small */
 int vs_format_sam(const vs_record *r, const char *qname, const char *rname, const uint8_t *guide,
                   const char *md, char *buf, size_t buflen);

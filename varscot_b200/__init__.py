@@ -11,9 +11,9 @@ from ._lib import VarscotError, GLEN
 _lib.lib()   # fail at import time, not at first use, when the CUDA library has not been built
 
 from .mapper import (PackedText, ScanContext, Mapper, bidir_index, bidir_mapping, vcf_loader, fasta_writer, device_count, format_sam, guide_codes,  # noqa: E402
-                     map_packed, map_records, md_string, merge_resolved, pam_code, records_key_set, resolve_hits, shard_bounds, HIT_DT, LOC_DT, REC_DT, BASES_DT, MASKS_DT, SPARSE_DT,
+                     map_packed, map_records, map_records_stream, md_from_window, md_string, merge_resolved, pam_code, records_key_set, resolve_hits, shard_bounds, HIT_DT, LOC_DT, REC_DT, BASES_DT, MASKS_DT, SPARSE_DT,
                      MD_SEQAN, MD_SAMTOOLS)
 
 __all__ = ["PackedText", "ScanContext", "Mapper", "bidir_index", "bidir_mapping", "vcf_loader", "fasta_writer", "device_count", "format_sam", "guide_codes",
-           "map_packed", "map_records", "md_string", "merge_resolved", "pam_code", "records_key_set", "resolve_hits", "shard_bounds", "VarscotError", "GLEN",
+           "map_packed", "map_records", "map_records_stream", "md_from_window", "md_string", "merge_resolved", "pam_code", "records_key_set", "resolve_hits", "shard_bounds", "VarscotError", "GLEN",
            "HIT_DT", "LOC_DT", "REC_DT", "BASES_DT", "MASKS_DT", "SPARSE_DT", "MD_SEQAN", "MD_SAMTOOLS"]

@@ -47,6 +47,7 @@ class LocHit(C.Structure):
 
 
 HIT_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32)
+RECORD_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32)
 VS_OPT_KEEP_INDEX, VS_OPT_HIT_CAPACITY, VS_OPT_BUCKET_INDEX = 1, 2, 3
 
 
@@ -70,8 +71,8 @@ EXPORTS = [
     "vs_ctx_create", "vs_ctx_destroy", "vs_last_error", "vs_ctx_set_chunk_words", "vs_text_upload", "vs_host_alloc",
     "vs_host_free", "vs_host_register", "vs_host_unregister", "vs_ctx_set_option", "vs_index_drop", "vs_scan", "vs_scan_text", "vs_scan_fetch",
     "vs_scan_resolved", "vs_merge_resolved", "vs_map_packed", "vs_shard_bounds", "vs_resolve_hits", "vs_resolve_hits_mt",
-    "vs_mapper_create", "vs_mapper_map", "vs_mapper_info", "vs_mapper_destroy",
-    "vs_md_string", "vs_format_sam", "vs_bidir_index_main", "vs_bidir_mapping_main", "vs_vcf_loader_main", "vs_fasta_writer_main", "vs_bam_merger_main", "vs_bam_merger_ref_only_main", "vs_measure_int_peaks",
+    "vs_mapper_create", "vs_mapper_map", "vs_mapper_info", "vs_mapper_destroy", "vs_mapper_map_stream", "vs_map_records_stream",
+    "vs_md_string", "vs_md_from_window", "vs_format_sam", "vs_bidir_index_main", "vs_bidir_mapping_main", "vs_vcf_loader_main", "vs_fasta_writer_main", "vs_bam_merger_main", "vs_bam_merger_ref_only_main", "vs_measure_int_peaks",
 ]
 
 _lib = None
@@ -124,11 +125,15 @@ def lib():
     L.vs_shard_bounds.argtypes = [u64, i32, vp]
     L.vs_mapper_create.argtypes = [C.POINTER(TextView), vp, i32, C.POINTER(vp)]
     L.vs_mapper_map.argtypes = [vp, vp, u32, i32, i32, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(ScanStats)]
+    L.vs_mapper_map_stream.argtypes = [vp, vp, u32, i32, i32, i32, u64, i32, RECORD_SINK, vp, C.POINTER(u64), C.POINTER(ScanStats)]
+    L.vs_map_records_stream.argtypes = [C.POINTER(TextView), vp, u32, i32, i32, vp, i32, i32, u64, i32, RECORD_SINK, vp, C.POINTER(u64),
+                                        C.POINTER(ScanStats)]
     L.vs_mapper_info.argtypes = [vp, C.POINTER(u32), C.POINTER(u64), C.POINTER(u64)]
     L.vs_mapper_destroy.argtypes = [vp]
     L.vs_resolve_hits.argtypes = [vp, u64, vp, u32, vp, C.POINTER(u64)]
     L.vs_resolve_hits_mt.argtypes = [vp, u64, vp, u32, vp, C.POINTER(u64), i32]
     L.vs_md_string.argtypes = [vp, u64, vp, i32, i32, C.c_char_p]
+    L.vs_md_from_window.argtypes = [u64, vp, i32, i32, C.c_char_p]
     L.vs_format_sam.argtypes = [C.POINTER(Record), C.c_char_p, C.c_char_p, vp, C.c_char_p, C.c_char_p, C.c_size_t]
     L.vs_bidir_index_main.argtypes = [i32, C.POINTER(C.c_char_p)]
     L.vs_bidir_mapping_main.argtypes = [i32, C.POINTER(C.c_char_p)]

@@ -381,71 +381,87 @@ extern "C" int vs_bidir_mapping_main(int argc, char **argv)
     FILE *out = fopen(output.c_str(), "wb");
     if (!out) { fprintf(stderr, "ERROR: Could not open output path.\n"); return 1; }
 
-    // the scan: every device resolves its hits to (contig, pos) and sorts them into the reference's emission order; the host
-    // merges the shards' lists and applies the primary / secondary rule.  -T drives the host side (merge, SAM formatting).
+    // the scan: every device resolves its hits to (contig, pos), sorts them into the reference's emission order and reads each
+    // hit's genome window; the host merges the shards' lists a range of guides at a time, applies the primary / secondary rule and
+    // formats the range's SAM on the -T host threads (MD:Z from the windows) while the devices score the next range.
+    // VARSCOT_RECORDS_PER_DELIVERY: records per range (0 = the library's default).
     const int host_threads = (int)std::min<long>(64, std::max<long>(1, threads));
-    std::vector<std::vector<vs_loc_hit>> lists;
     const uint32_t n_guides = (uint32_t)ids.size();
+    struct Writer {
+        FILE *out;
+        const std::vector<std::string> &ids, &names;
+        const std::vector<uint8_t> &guides;
+        int md_style, host_threads;
+        bool write_failed = false;
+        uint64_t deliveries = 0, largest = 0;
+        std::vector<std::string> parts;
+        // SAM text: batches of records are formatted by the host threads into per-thread buffers and written in order
+        int write(const vs_record *rec, const uint64_t *win, uint64_t n)
+        {
+            ++deliveries;
+            largest = std::max(largest, n);
+            const size_t batch = (size_t)host_threads * 65536;
+            parts.resize((size_t)host_threads);
+            for (size_t b0 = 0; b0 < n; b0 += batch) {
+                const size_t b1 = std::min<size_t>(n, b0 + batch);
+                auto format = [&](int ti) {
+                    std::string &o = parts[(size_t)ti];
+                    o.clear();
+                    const size_t r0 = b0 + (b1 - b0) * (size_t)ti / (size_t)host_threads, r1 = b0 + (b1 - b0) * (size_t)(ti + 1) / (size_t)host_threads;
+                    std::vector<char> buf(1 << 12);
+                    for (size_t i = r0; i < r1; ++i) {
+                        const vs_record &r = rec[i];
+                        char md[64];
+                        const uint8_t *g = guides.data() + (size_t)r.guide * VS_GLEN;
+                        vs_md_from_window(win[i], g, (r.flag >> 4) & 1, md_style, md);
+                        const std::string &qn = ids[r.guide], &rn = names[r.contig];
+                        if (buf.size() < qn.size() + rn.size() + 256) buf.resize(qn.size() + rn.size() + 256);
+                        int len = vs_format_sam(&r, qn.c_str(), rn.c_str(), g, md, buf.data(), buf.size());
+                        if (len > 0) o.append(buf.data(), (size_t)len);
+                    }
+                };
+                if (host_threads == 1) format(0);
+                else {
+                    std::vector<std::thread> th;
+                    for (int ti = 0; ti < host_threads; ++ti) th.emplace_back(format, ti);
+                    for (auto &x : th) x.join();
+                }
+                for (const std::string &o : parts)
+                    if (!o.empty() && fwrite(o.data(), 1, o.size(), out) != o.size()) { write_failed = true; return 1; }
+            }
+            return 0;
+        }
+        static int sink(void *user, const vs_record *rec, const uint64_t *win, uint64_t n, uint32_t, uint32_t)
+        {
+            return static_cast<Writer *>(user)->write(rec, win, n);
+        }
+    } writer{out, ids, t.names, guides, md_style, host_threads};
+    uint64_t coll = 0;
     if (n_guides && t.v.n_bases) {
         std::vector<int> devices = choose_devices(t.v.n_bases);
         if (devices.empty()) { fprintf(stderr, "%s: no usable CUDA device: %s (this build has no CPU path)\n", prog, vs_last_error(nullptr)); fclose(out); return 1; }
+        const char *rpd = getenv("VARSCOT_RECORDS_PER_DELIVERY");
         vs_scan_stats st;
-        int rc = vs::scan_text_sharded_resolved(t.v, devices, guides.data(), n_guides, (int)mism, extra_pam, lists, &st, err);
-        if (rc != VS_OK) { fprintf(stderr, "%s: scan failed: %s\n", prog, err.c_str()); fclose(out); return 1; }
+        int rc = vs_map_records_stream(&t.v, guides.data(), n_guides, (int)mism, extra_pam, devices.data(), (int)devices.size(), host_threads,
+                                       rpd ? strtoull(rpd, nullptr, 10) : 0, 1, &Writer::sink, &writer, &coll, &st);
+        if (writer.write_failed) { fprintf(stderr, "%s: write error\n", prog); fclose(out); return 1; }
+        if (rc != VS_OK) { fprintf(stderr, "%s: scan failed: %s\n", prog, vs_last_error(nullptr)); fclose(out); return 1; }
         if (getenv("VARSCOT_VERBOSE"))
             for (int dv : devices) fprintf(stderr, "%s: scanning on device %d\n", prog, dv);
         if (getenv("VARSCOT_VERBOSE"))
-            fprintf(stderr, "%s: %zu device(s), %.3f ms upload+scan (extract %.3f, score %.3f, resolve+sort %.3f; %.1f MB H2D), %llu candidates, %llu hits\n", prog,
+            fprintf(stderr, "%s: %zu device(s), %.3f ms upload+scan (extract %.3f, score %.3f, resolve+sort %.3f; %.1f MB H2D), %llu candidates, %llu hits, "
+                            "%llu deliveries (largest %llu records)\n", prog,
                     devices.size(), st.total_ms, st.extract_ms, st.score_ms, st.resolve_ms, st.h2d_bytes / 1e6,
-                    (unsigned long long)(st.n_cand_fwd + st.n_cand_rev), (unsigned long long)st.n_hits);
+                    (unsigned long long)(st.n_cand_fwd + st.n_cand_rev), (unsigned long long)st.n_hits, (unsigned long long)writer.deliveries,
+                    (unsigned long long)writer.largest);
     }
     const auto tm2 = std::chrono::steady_clock::now();
-    std::vector<const vs_loc_hit *> lp;
-    std::vector<uint64_t> lc;
-    uint64_t n_rec = 0;
-    for (auto &l : lists) { lp.push_back(l.data()); lc.push_back(l.size()); n_rec += l.size(); }
-    std::vector<vs_record> rec(n_rec);
-    uint64_t coll = 0;
-    if (n_rec && vs_merge_resolved(lp.data(), lc.data(), (int)lp.size(), rec.data(), &coll, host_threads) != VS_OK) {
-        fprintf(stderr, "%s: %s\n", prog, vs_last_error(nullptr)); fclose(out); return 1;
-    }
-    lists.clear();
     if (coll) fprintf(stderr, "%s: note: %llu records share a (contig id mod 65536, position) key; the reference's uint16 map key would have kept one of each\n", prog, (unsigned long long)coll);
-    // SAM text: batches of records are formatted by the host threads into per-thread buffers and written in order
-    const size_t batch = (size_t)host_threads * 65536;
-    std::vector<std::string> parts((size_t)host_threads);
-    for (size_t b0 = 0; b0 < rec.size(); b0 += batch) {
-        const size_t b1 = std::min(rec.size(), b0 + batch);
-        auto format = [&](int ti) {
-            std::string &o = parts[(size_t)ti];
-            o.clear();
-            const size_t r0 = b0 + (b1 - b0) * (size_t)ti / (size_t)host_threads, r1 = b0 + (b1 - b0) * (size_t)(ti + 1) / (size_t)host_threads;
-            std::vector<char> buf(1 << 12);
-            for (size_t i = r0; i < r1; ++i) {
-                const vs_record &r = rec[i];
-                char md[64];
-                const uint8_t *g = guides.data() + (size_t)r.guide * VS_GLEN;
-                vs_md_string(t.v.bases, t.v.contig_off[r.contig] + r.pos, g, (r.flag >> 4) & 1, md_style, md);
-                const std::string &qn = ids[r.guide], &rn = t.names[r.contig];
-                if (buf.size() < qn.size() + rn.size() + 256) buf.resize(qn.size() + rn.size() + 256);
-                int n = vs_format_sam(&r, qn.c_str(), rn.c_str(), g, md, buf.data(), buf.size());
-                if (n > 0) o.append(buf.data(), (size_t)n);
-            }
-        };
-        if (host_threads == 1) format(0);
-        else {
-            std::vector<std::thread> th;
-            for (int ti = 0; ti < host_threads; ++ti) th.emplace_back(format, ti);
-            for (auto &x : th) x.join();
-        }
-        for (const std::string &o : parts)
-            if (!o.empty() && fwrite(o.data(), 1, o.size(), out) != o.size()) { fprintf(stderr, "%s: write error\n", prog); fclose(out); return 1; }
-    }
     if (fclose(out) != 0) { fprintf(stderr, "%s: write error\n", prog); return 1; }
     if (getenv("VARSCOT_VERBOSE")) {
         auto sec = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double>(b - a).count(); };
-        fprintf(stderr, "%s: wall: load %.3f s, device (context + upload + scan) %.3f s, resolve + SAM %.3f s\n", prog, sec(tm0, tm1), sec(tm1, tm2),
-                sec(tm2, std::chrono::steady_clock::now()));
+        fprintf(stderr, "%s: wall: load %.3f s, device (context + upload + scan) overlapped with resolve + SAM %.3f s, close %.3f s\n", prog,
+                sec(tm0, tm1), sec(tm1, tm2), sec(tm2, std::chrono::steady_clock::now()));
     }
     return 0;
 }

@@ -118,6 +118,8 @@ struct vs_ctx {
     Buf<vs_loc_hit> d_loc;
     PinnedBuf<vs_loc_hit> h_stage;
     Buf<uint8_t> d_sort_tmp;
+    Buf<uint64_t> d_win;                 // genome windows of the sorted hits (scans that ask for them) and their staging
+    PinnedBuf<uint64_t> h_win;
     std::string err;
 };
 
@@ -744,6 +746,13 @@ static double hit_density(int k, int n_pam)
     return 2.0 * n_pam / 16.0 * p;
 }
 
+double vs::expected_hits_per_base(int k, int extra_pam)
+{
+    PamParams pp;
+    make_pam(extra_pam, pp);
+    return hit_density(k, pp.n);
+}
+
 // ---- bucketed index (vs_bucket.cuh) --------------------------------------------------------------------------------
 // Built from the resident plain index and the resident text: bucket histogram -> padded bucket starts -> positions
 // regrouped by bucket -> blocks gathered from the text.  Two host synchronisations: the store is sized by the padded total
@@ -817,7 +826,8 @@ struct Scan {
     vs_loc_hit *out_loc = nullptr;
     uint64_t out_cap = 0;
     uint64_t *n_hits = nullptr;
-    vs_hit_sink sink = nullptr;
+    bool windows = false;                    // resolved: the genome window of every hit too (k_loc_windows)
+    loc_sink sink = nullptr;
     void *user = nullptr;
     vs_scan_stats *stats = nullptr;
     Upload up;                               // the text from the host: not resident while up.t is set
@@ -1042,6 +1052,16 @@ static int deliver(vs_ctx *ctx, Scan &s, uint32_t g0, uint32_t ng, uint64_t foun
         k_pack_loc_hits<<<gb, 256, 0, st>>>(dk.Current(), dv.Current(), found, ctx->d_loc);
         s.S.launches += 2 + 8;                              // + the radix sort's passes (CUB: histogram + one pass per 8 key bits)
         CK(cudaGetLastError());
+        if (s.windows) {
+            if (found > ctx->d_win.cap && (ctx->d_win.grow(ctx, found + found / 8) || ctx->h_win.grow(ctx, found + found / 8)))
+                return release_all(ctx->d_win, ctx->h_win);
+            k_loc_windows<<<gb, 256, 0, st>>>(ctx->d_loc, found, ctx->d_cstart, ctx->text.first_contig, ctx->d_bases,
+                                              ctx->text.first_word * 32 - ctx->text.pos_origin, ctx->d_win);
+            s.S.launches++;
+            CK(cudaGetLastError());
+            CK(cudaMemcpyAsync(ctx->h_win, ctx->d_win, found * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            s.S.d2h_bytes += found * sizeof(uint64_t);
+        }
         if (s.sink) {
             if (found > ctx->h_stage.cap && (r = ctx->h_stage.grow(ctx, found + found / 8)) != VS_OK) return r;
             CK(cudaMemcpyAsync(ctx->h_stage, ctx->d_loc, found * sizeof(vs_loc_hit), cudaMemcpyDeviceToHost, st));
@@ -1056,7 +1076,7 @@ static int deliver(vs_ctx *ctx, Scan &s, uint32_t g0, uint32_t ng, uint64_t foun
     float a = 0.f;
     CK(cudaEventElapsedTime(&a, ctx->t0[vs_ctx::T_DELIVER], ctx->t1[vs_ctx::T_DELIVER]));
     s.S.resolve_ms += a;
-    if (s.resolved && s.sink && found && s.sink(s.user, ctx->h_stage, found, g0, g0 + ng) != 0)
+    if (s.resolved && s.sink && found && s.sink(s.user, ctx->h_stage, s.windows ? ctx->h_win.p : nullptr, found, g0, g0 + ng) != 0)
         return fail(ctx, VS_ERR_ARG, "vs_scan_resolved: the sink aborted the scan");
     return VS_OK;
 }
@@ -1198,9 +1218,9 @@ extern "C" int vs_scan_text(vs_ctx *ctx, const vs_text_view *text, uint64_t firs
     return scan_engine(ctx, q);
 }
 
-extern "C" int vs_scan_resolved(vs_ctx *ctx, const vs_text_view *text, uint64_t first_word, uint64_t n_words,
-                                const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
-                                vs_loc_hit *out, uint64_t out_cap, uint64_t *n_hits, vs_hit_sink sink, void *user, vs_scan_stats *stats)
+int vs::scan_resolved_ex(vs_ctx *ctx, const vs_text_view *text, uint64_t first_word, uint64_t n_words,
+                         const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
+                         vs_loc_hit *out, uint64_t out_cap, uint64_t *n_hits, bool windows, loc_sink sink, void *user, vs_scan_stats *stats)
 {
     if (!ctx) return fail(nullptr, VS_ERR_ARG, "vs_scan_resolved: ctx is NULL");
     if (text) {
@@ -1210,8 +1230,30 @@ extern "C" int vs_scan_resolved(vs_ctx *ctx, const vs_text_view *text, uint64_t 
     Scan q;
     q.src = text; q.first_word = first_word; q.n_words = n_words;
     q.guides = guides; q.n_guides = n_guides; q.k = k; q.extra_pam = extra_pam;
-    q.resolved = true; q.out_loc = out; q.out_cap = out_cap; q.n_hits = n_hits; q.sink = sink; q.user = user; q.stats = stats;
+    q.resolved = true; q.out_loc = out; q.out_cap = out_cap; q.n_hits = n_hits; q.stats = stats;
+    q.windows = windows; q.sink = sink; q.user = user;
     return scan_engine(ctx, q);
+}
+
+namespace {
+struct PublicSink {
+    vs_hit_sink sink;
+    void *user;
+    static int call(void *u, const vs_loc_hit *h, const uint64_t *, uint64_t n, uint32_t g0, uint32_t g1)
+    {
+        const PublicSink *p = static_cast<const PublicSink *>(u);
+        return p->sink(p->user, h, n, g0, g1);
+    }
+};
+}  // namespace
+
+extern "C" int vs_scan_resolved(vs_ctx *ctx, const vs_text_view *text, uint64_t first_word, uint64_t n_words,
+                                const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
+                                vs_loc_hit *out, uint64_t out_cap, uint64_t *n_hits, vs_hit_sink sink, void *user, vs_scan_stats *stats)
+{
+    PublicSink p{sink, user};
+    return scan_resolved_ex(ctx, text, first_word, n_words, guides, n_guides, k, extra_pam, out, out_cap, n_hits, false,
+                            sink ? &PublicSink::call : nullptr, &p, stats);
 }
 
 extern "C" int vs_scan_fetch(vs_ctx *ctx, vs_hit *out, uint64_t out_cap, uint64_t *n_hits)

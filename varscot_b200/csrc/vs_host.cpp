@@ -6,6 +6,7 @@
 #include "vs_internal.h"
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <emmintrin.h>
 #include <cstdio>
 #include <cstdlib>
@@ -576,8 +577,10 @@ extern "C" int vs_resolve_hits(const vs_hit *hits, uint64_t n, const uint64_t *c
 // into its final place in `out`'s index space, sorted when more than one list contributed (or when records tie on the
 // 16-bit key: the order among those is by the full contig id), and walked with the running-best rule of
 // bidir_mapping.cpp:164-187.
-extern "C" int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t *counts, int n_lists,
-                                 vs_record *out, uint64_t *key16_collisions, int n_threads)
+// wins (optional): one window per hit of every list, moved through the same permutation into win_out; guide_base is added to
+// every record's guide id
+static int merge_impl(const vs_loc_hit *const *lists, const uint64_t *counts, const uint64_t *const *wins, int n_lists, uint32_t guide_base,
+                      vs_record *out, uint64_t *win_out, uint64_t *key16_collisions, int n_threads)
 {
     if (key16_collisions) *key16_collisions = 0;
     if (n_lists < 0 || (n_lists && (!lists || !counts))) return VS_ERR_ARG;
@@ -615,16 +618,20 @@ extern "C" int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t 
     auto work = [&](int t) {
         const uint64_t o0 = out_at[(size_t)t], o1 = out_at[(size_t)t + 1];
         if (o1 == o0) return;
-        struct Head { const vs_loc_hit *p, *e; };
+        // a hit and its window (null without windows): what the walk holds back moves with its window
+        struct Item { const vs_loc_hit *h; const uint64_t *win; };
+        struct Head { const vs_loc_hit *p, *e; const uint64_t *win; };
         std::vector<Head> heads;
         for (int l = 0; l < n_lists; ++l) {
-            const vs_loc_hit *b = lists[l] + at[(size_t)t * (size_t)n_lists + (size_t)l], *e = lists[l] + at[(size_t)(t + 1) * (size_t)n_lists + (size_t)l];
-            if (b < e) heads.push_back(Head{b, e});
+            const uint64_t i0 = at[(size_t)t * (size_t)n_lists + (size_t)l], i1 = at[(size_t)(t + 1) * (size_t)n_lists + (size_t)l];
+            if (i0 < i1) heads.push_back(Head{lists[l] + i0, lists[l] + i1, wins ? wins[l] + i0 : nullptr});
         }
         uint64_t w = o0, c = 0;
-        auto emit = [&](const vs_loc_hit &h, uint16_t secondary) {
+        auto emit = [&](const Item &it, uint16_t secondary) {
+            const vs_loc_hit &h = *it.h;
+            if (win_out) win_out[w] = *it.win;
             vs_record &o = out[w++];
-            o.guide = h.info >> 8;
+            o.guide = (h.info >> 8) + guide_base;
             o.contig = h.contig;
             o.pos = (uint32_t)h.key;
             o.mm = (uint8_t)(h.info & 0x7F);
@@ -633,41 +640,42 @@ extern "C" int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t 
         };
         // running-best walk (bidir_mapping.cpp:164-187), fed one record at a time in emission-key order
         bool have_best = false;
-        vs_loc_hit best{};
+        Item best{};
         uint64_t cur_pass = ~0ull;
-        auto feed = [&](const vs_loc_hit &h) {
-            const uint64_t p = pass_of(h);
+        auto feed = [&](const Item &it) {
+            const uint64_t p = pass_of(*it.h);
             if (p != cur_pass) {
                 if (have_best) emit(best, 0);
-                best = h; have_best = true; cur_pass = p;
+                best = it; have_best = true; cur_pass = p;
                 return;
             }
-            if ((h.info & 0x7F) >= (best.info & 0x7F)) emit(h, 256);
-            else { emit(best, 256); best = h; }
+            if ((it.h->info & 0x7F) >= (best.h->info & 0x7F)) emit(it, 256);
+            else { emit(best, 256); best = it; }
         };
         // records sharing (pass, strand, contig & 0xFFFF, pos) — a uint16 key collision, rare — are ordered by the full contig id:
         // one record is held back until the next one shows a different key
-        std::vector<vs_loc_hit> ties;
+        std::vector<Item> ties;
         bool have_prev = false;
-        vs_loc_hit prev{};
+        Item prev{};
         uint64_t prev_pass = 0, prev_key = 0;
         auto flush_ties = [&]() {
             if (!ties.empty()) {
                 ties.push_back(prev);
-                std::sort(ties.begin(), ties.end(), [](const vs_loc_hit &a, const vs_loc_hit &b) { return a.contig < b.contig; });
+                std::sort(ties.begin(), ties.end(), [](const Item &a, const Item &b) { return a.h->contig < b.h->contig; });
                 c += ties.size() - 1;
-                for (const vs_loc_hit &h : ties) feed(h);
+                for (const Item &it : ties) feed(it);
                 ties.clear();
             } else if (have_prev) feed(prev);
             have_prev = false;
         };
-        auto take = [&](const vs_loc_hit &h, uint64_t p, uint64_t k) {
-            if (have_prev && p == prev_pass && k == prev_key) { ties.push_back(prev); prev = h; return; }
+        auto take = [&](const Item &it, uint64_t p, uint64_t k) {
+            if (have_prev && p == prev_pass && k == prev_key) { ties.push_back(prev); prev = it; return; }
             flush_ties();
-            prev = h; prev_pass = p; prev_key = k; have_prev = true;
+            prev = it; prev_pass = p; prev_key = k; have_prev = true;
         };
         if (heads.size() == 1) {
-            for (const vs_loc_hit *p = heads[0].p; p < heads[0].e; ++p) take(*p, pass_of(*p), p->key & KEY48);
+            const Head &hd = heads[0];
+            for (const vs_loc_hit *p = hd.p; p < hd.e; ++p) take(Item{p, hd.win ? hd.win + (p - hd.p) : nullptr}, pass_of(*p), p->key & KEY48);
         } else {
             // k-way merge by linear selection over the cached keys of the heads (k = number of shards, a handful)
             const size_t k = heads.size();
@@ -678,8 +686,10 @@ extern "C" int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t 
                 size_t m = 0;
                 for (size_t i = 1; i < k; ++i)
                     if (hp[i] < hp[m] || (hp[i] == hp[m] && hk[i] < hk[m])) m = i;
-                take(*heads[m].p, hp[m], hk[m]);
-                if (++heads[m].p < heads[m].e) { hp[m] = pass_of(*heads[m].p); hk[m] = heads[m].p->key & KEY48; }
+                Head &hd = heads[m];
+                take(Item{hd.p, hd.win}, hp[m], hk[m]);
+                if (hd.win) ++hd.win;
+                if (++hd.p < hd.e) { hp[m] = pass_of(*hd.p); hk[m] = hd.p->key & KEY48; }
                 else { hp[m] = ~0ull; hk[m] = ~0ull; --live; }
             }
         }
@@ -699,22 +709,22 @@ extern "C" int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t 
     return VS_OK;
 }
 
-static inline int base_at(const vs_bases *bases, uint64_t p)
+extern "C" int vs_merge_resolved(const vs_loc_hit *const *lists, const uint64_t *counts, int n_lists,
+                                 vs_record *out, uint64_t *key16_collisions, int n_threads)
 {
-    const vs_bases &w = bases[p >> 5];
-    uint32_t b = (uint32_t)(p & 31);
-    return (int)(((w.hi >> b) & 1) << 1 | ((w.lo >> b) & 1));     // hits never contain N
+    return merge_impl(lists, counts, nullptr, n_lists, 0, out, nullptr, key16_collisions, n_threads);
 }
 
-extern "C" int vs_md_string(const vs_bases *words, uint64_t gpos, const uint8_t *guide, int strand, int md_style, char *out)
+// MD:Z of the window whose base i is base(i) (bidir_mapping.cpp:111-123)
+template <class Base>
+static void md_of(Base base, const uint8_t *guide, int strand, int md_style, char *out)
 {
-    if (!words || !guide || !out) return VS_ERR_ARG;
     static const char L[4] = {'A', 'C', 'G', 'T'};
     int n = 0, run = 0;
     bool in_match = false, any = false;
     for (int i = 0; i < VS_GLEN; ++i) {
         int g = strand ? 3 - guide[VS_GLEN - 1 - i] : guide[i];   // pattern of the pass, genome-forward orientation
-        int t = base_at(words, gpos + i);
+        int t = base(i);
         if (t == g) { ++run; in_match = true; any = true; continue; }
         // mismatch column: genome character (row 0 of the Align at bidir_mapping.cpp:117)
         if (md_style == VS_MD_SAMTOOLS) n += sprintf(out + n, "%d", run);
@@ -725,6 +735,24 @@ extern "C" int vs_md_string(const vs_bases *words, uint64_t gpos, const uint8_t 
     if (md_style == VS_MD_SAMTOOLS || in_match) n += sprintf(out + n, "%d", run);
     (void)any;
     out[n] = 0;
+}
+
+extern "C" int vs_md_string(const vs_bases *words, uint64_t gpos, const uint8_t *guide, int strand, int md_style, char *out)
+{
+    if (!words || !guide || !out) return VS_ERR_ARG;
+    md_of([&](int i) {
+        const uint64_t p = gpos + (uint64_t)i;
+        const vs_bases &w = words[p >> 5];
+        const uint32_t b = (uint32_t)(p & 31);
+        return (int)(((w.hi >> b) & 1) << 1 | ((w.lo >> b) & 1));     // hits never contain N
+    }, guide, strand, md_style, out);
+    return VS_OK;
+}
+
+extern "C" int vs_md_from_window(uint64_t window, const uint8_t *guide, int strand, int md_style, char *out)
+{
+    if (!guide || !out) return VS_ERR_ARG;
+    md_of([&](int i) { return (int)((window >> (2 * i)) & 3); }, guide, strand, md_style, out);
     return VS_OK;
 }
 
@@ -839,31 +867,180 @@ static int for_each_shard(const std::vector<uint64_t> &b, const std::vector<int>
     return VS_OK;
 }
 
-// the sink of vs_scan_resolved that appends every super-chunk to a std::vector<vs_loc_hit>
-static int append_sink(void *user, const vs_loc_hit *h, uint64_t n, uint32_t, uint32_t)
+// ---- guide-range streaming ----
+uint64_t RangeLists::total() const
 {
-    auto *v = static_cast<std::vector<vs_loc_hit> *>(user);
-    try { v->insert(v->end(), h, h + n); } catch (...) { return 1; }
-    return 0;
+    uint64_t n = 0;
+    for (const auto &h : hits) n += h.size();
+    return n;
 }
 
-// the shard lists of vs_scan_resolved -> records in emission order (malloc'd; NULL when there are none)
-static int merge_lists(const std::vector<std::vector<vs_loc_hit>> &lists, int n_threads, vs_record **records, uint64_t *n_records,
-                       uint64_t *key16_collisions)
+uint32_t next_range_guides(uint64_t target, double per_guide, uint32_t left)
 {
-    std::vector<const vs_loc_hit *> ptr;
-    std::vector<uint64_t> cnt;
-    uint64_t total = 0;
-    for (auto &l : lists) { ptr.push_back(l.data()); cnt.push_back(l.size()); total += l.size(); }
-    if (key16_collisions) *key16_collisions = 0;
-    if (total == 0) return VS_OK;
-    vs_record *o = (vs_record *)malloc(total * sizeof(vs_record));
-    if (!o) return VS_ERR_NOMEM;
-    const int rc = vs_merge_resolved(ptr.data(), cnt.data(), (int)ptr.size(), o, key16_collisions, n_threads);
-    if (rc != VS_OK) { free(o); return rc; }
-    *records = o; *n_records = total;
+    if (target == UINT64_MAX || per_guide <= 0) return left;
+    const double g = std::floor((double)target / per_guide);
+    return g >= (double)left ? left : std::max<uint32_t>(1, (uint32_t)g);
+}
+
+int stream_ranges(uint32_t n_guides, uint64_t target, double first_per_guide, const RangeScan &scan, const RangeDeliver &deliver,
+                  vs_scan_stats *stats, std::string &err)
+{
+    if (stats) memset(stats, 0, sizeof(*stats));
+    RangeLists lists[2];
+    vs_scan_stats st[2];
+    bool first = true;
+    auto add = [&](const vs_scan_stats &s) {              // ranges run one after the other: times and passes add up
+        if (!stats) return;
+        const uint32_t passes = stats->guide_passes;
+        add_stats(stats, s, true, first);
+        stats->guide_passes = passes + s.guide_passes;
+        first = false;
+    };
+    auto guarded_scan = [&](uint32_t lo, uint32_t hi, RangeLists &l, vs_scan_stats *s, std::string &e) {
+        memset(s, 0, sizeof(*s));
+        try { return scan(lo, hi, l, s, e); } catch (...) { e = "out of host memory"; return (int)VS_ERR_NOMEM; }
+    };
+    uint32_t lo = 0, hi = next_range_guides(target, first_per_guide, n_guides);
+    int r = guarded_scan(lo, hi, lists[0], &st[0], err);
+    if (r != VS_OK) return r;
+    add(st[0]);
+    for (int c = 0;; c ^= 1) {
+        // the next range, sized from the hits per guide of the range just scanned, is scanned while this one is delivered
+        const uint64_t got = lists[c].total();
+        const uint32_t nlo = hi, nhi = nlo + next_range_guides(target, hi > lo ? (double)std::max<uint64_t>(got, 1) / (hi - lo) : first_per_guide, n_guides - nlo);
+        int rs = VS_OK, rd = VS_OK;
+        std::string es;
+        std::thread next;
+        if (nlo < n_guides) next = std::thread([&] { rs = guarded_scan(nlo, nhi, lists[c ^ 1], &st[c ^ 1], es); });
+        try { rd = deliver(lists[c], lo, hi, err); } catch (...) { err = "out of host memory"; rd = VS_ERR_NOMEM; }
+        if (next.joinable()) next.join();
+        if (rd != VS_OK) return rd;
+        if (nlo >= n_guides) return VS_OK;
+        if (rs != VS_OK) { err = es; return rs; }
+        add(st[c ^ 1]);
+        lo = nlo; hi = nhi;
+    }
+}
+
+// first index of a sorted list whose guide (relative to the range) is >= g
+static uint64_t guide_start(const std::vector<vs_loc_hit> &l, uint32_t g)
+{
+    return (uint64_t)(std::partition_point(l.begin(), l.end(), [g](const vs_loc_hit &h) { return (h.info >> 8) < g; }) - l.begin());
+}
+
+uint64_t range_count(const RangeLists &lists, uint32_t g_lo, uint32_t g_hi)
+{
+    uint64_t n = 0;
+    for (const auto &l : lists.hits) n += guide_start(l, g_hi) - guide_start(l, g_lo);
+    return n;
+}
+
+int merge_range(const RangeLists &lists, uint32_t g_lo, uint32_t g_hi, uint32_t guide_base, vs_record *out, uint64_t *win_out,
+                uint64_t *key16_collisions, int n_threads)
+{
+    const size_t n = lists.hits.size();
+    std::vector<const vs_loc_hit *> ptr(n);
+    std::vector<const uint64_t *> win(n);
+    std::vector<uint64_t> cnt(n);
+    for (size_t s = 0; s < n; ++s) {
+        const uint64_t a = guide_start(lists.hits[s], g_lo), b = guide_start(lists.hits[s], g_hi);
+        ptr[s] = lists.hits[s].data() + a;
+        cnt[s] = b - a;
+        win[s] = win_out && !lists.win[s].empty() ? lists.win[s].data() + a : nullptr;
+        if (win_out && cnt[s] && !win[s]) return VS_ERR_ARG;
+    }
+    return merge_impl(ptr.data(), cnt.data(), win_out ? win.data() : nullptr, (int)n, guide_base, out, win_out, key16_collisions, n_threads);
+}
+
+int deliver_pieces(const RangeLists &lists, uint32_t lo, uint32_t hi, uint64_t target, bool windows, int n_threads,
+                   vs_record_sink sink, void *user, std::vector<vs_record> &rec, std::vector<uint64_t> &win, uint64_t *key16_collisions)
+{
+    const uint32_t n = hi - lo;
+    if (rec.empty()) rec.resize(1);                         // the sink gets non-null pointers, windows whenever asked for
+    if (windows && win.empty()) win.resize(1);
+    if (n == 0) return sink(user, rec.data(), windows ? win.data() : nullptr, 0, lo, hi) ? SINK_ABORTED : VS_OK;
+    for (uint32_t a = 0; a < n;) {
+        // the most whole guides from a on that stay within the target; at least one
+        uint32_t b = a + 1;
+        if (range_count(lists, a, n) <= target) b = n;
+        else {
+            uint32_t x = a + 1, y = n;                      // count(a, x) may exceed the target; count(a, y) does
+            while (y - x > 1) {
+                const uint32_t mid = x + (y - x) / 2;
+                if (range_count(lists, a, mid) <= target) x = mid; else y = mid;
+            }
+            b = x;
+        }
+        const uint64_t cnt = range_count(lists, a, b);
+        if (rec.size() < cnt) rec.resize(cnt);
+        if (windows && win.size() < cnt) win.resize(cnt);
+        uint64_t c = 0;
+        const int r = merge_range(lists, a, b, lo, rec.data(), windows ? win.data() : nullptr, &c, n_threads);
+        if (r != VS_OK) return r;
+        *key16_collisions += c;
+        if (sink(user, rec.data(), windows ? win.data() : nullptr, cnt, lo + a, lo + b) != 0) return SINK_ABORTED;
+        a = b;
+    }
     return VS_OK;
 }
+
+// the sink of scan_resolved_ex that appends every super-chunk of a shard to its lists
+namespace {
+struct Collect {
+    std::vector<vs_loc_hit> *hits;
+    std::vector<uint64_t> *win;
+    static int sink(void *user, const vs_loc_hit *h, const uint64_t *w, uint64_t n, uint32_t, uint32_t)
+    {
+        const Collect *c = static_cast<const Collect *>(user);
+        try {
+            c->hits->insert(c->hits->end(), h, h + n);
+            if (w) c->win->insert(c->win->end(), w, w + n);
+        } catch (...) { return 1; }
+        return 0;
+    }
+};
+}  // namespace
+
+static void reset_lists(RangeLists &l, size_t n_shards)
+{
+    l.hits.resize(n_shards);
+    l.win.resize(n_shards);
+    for (size_t s = 0; s < n_shards; ++s) { l.hits[s].clear(); l.win[s].clear(); }
+}
+
+// One unlimited range merged straight into a malloc'd array (vs_mapper_map, vs_map_records): NULL when there are no records.
+static RangeDeliver merge_all(int n_threads, vs_record **records, uint64_t *n_records, uint64_t *key16_collisions)
+{
+    return [=](const RangeLists &lists, uint32_t lo, uint32_t hi, std::string &) {
+        if (key16_collisions) *key16_collisions = 0;
+        const uint64_t total = lists.total();
+        if (total == 0) return (int)VS_OK;
+        vs_record *o = (vs_record *)malloc(total * sizeof(vs_record));
+        if (!o) return (int)VS_ERR_NOMEM;
+        const int rc = merge_range(lists, 0, hi - lo, lo, o, nullptr, key16_collisions, n_threads);
+        if (rc != VS_OK) { free(o); return rc; }
+        *records = o; *n_records = total;
+        return (int)VS_OK;
+    };
+}
+
+// A vs_record_sink fed piece by piece (vs_mapper_map_stream, vs_map_records_stream)
+struct SinkDeliver {
+    uint64_t target;
+    bool windows;
+    int n_threads;
+    vs_record_sink sink;
+    void *user;
+    uint64_t collisions = 0;
+    std::vector<vs_record> rec;
+    std::vector<uint64_t> win;
+    int operator()(const RangeLists &lists, uint32_t lo, uint32_t hi, std::string &err)
+    {
+        const int r = deliver_pieces(lists, lo, hi, target, windows, n_threads, sink, user, rec, win, &collisions);
+        if (r == SINK_ABORTED) { err = "the sink aborted"; return VS_ERR_ARG; }
+        return r;
+    }
+};
 
 static std::vector<int> or_device0(const std::vector<int> &devices) { return devices.empty() ? std::vector<int>{0} : devices; }
 
@@ -893,19 +1070,36 @@ int scan_text_sharded(const vs_text_view &text, const std::vector<int> &devices_
     return VS_OK;
 }
 
-// the same with the hits resolved and sorted on every device (vs_scan_resolved): one list per shard, ready for vs_merge_resolved
-int scan_text_sharded_resolved(const vs_text_view &text, const std::vector<int> &devices_in,
-                               const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
-                               std::vector<std::vector<vs_loc_hit>> &lists, vs_scan_stats *agg, std::string &err)
+// vs_map_records(_stream): the text from the host, sharded as shard_plan.  With one shard per device every device keeps one
+// context for the whole call: the first range streams the upload and extracts the index, later ranges score it.  With several
+// shards per device every range gets fresh contexts and uploads every shard again.
+static int map_text(const vs_text_view &text, const std::vector<int> &devices_in, const uint8_t *guides, uint32_t n_guides, int k,
+                    int extra_pam, uint64_t target, bool windows, const RangeDeliver &deliver, vs_scan_stats *stats, std::string &err)
 {
     const std::vector<int> devices = or_device0(devices_in);
     const std::vector<uint64_t> b = shard_plan(text.n_words, (int)devices.size());
-    lists.assign(b.size() - 1, {});
-    return for_each_shard(b, devices, nullptr, agg, err, [&](int i, vs_ctx *ctx, uint64_t w0, uint64_t n, vs_scan_stats *st) {
-        uint64_t cnt = 0;
-        vs_ctx_set_option(ctx, VS_OPT_KEEP_INDEX, 0);
-        return vs_scan_resolved(ctx, &text, w0, n, guides, n_guides, k, extra_pam, nullptr, 0, &cnt, &append_sink, &lists[(size_t)i], st);
-    });
+    const size_t n_shards = b.size() - 1;
+    const bool keep = n_shards == devices.size();
+    std::vector<vs_ctx *> ctx(keep ? n_shards : 0, nullptr);
+    bool uploaded = false;
+    const RangeScan scan = [&](uint32_t lo, uint32_t hi, RangeLists &lists, vs_scan_stats *st, std::string &e) {
+        reset_lists(lists, n_shards);
+        const int r = for_each_shard(b, devices, keep ? &ctx : nullptr, st, e, [&](int s, vs_ctx *c, uint64_t w0, uint64_t n, vs_scan_stats *st1) {
+            uint64_t cnt = 0;
+            Collect col{&lists.hits[(size_t)s], &lists.win[(size_t)s]};
+            vs_ctx_set_option(c, VS_OPT_KEEP_INDEX, keep ? 1 : 0);
+            return scan_resolved_ex(c, keep && uploaded ? nullptr : &text, w0, n, guides + (size_t)lo * VS_GLEN, hi - lo, k, extra_pam,
+                                    nullptr, 0, &cnt, windows, &Collect::sink, &col, st1);
+        });
+        uploaded = true;
+        return r;
+    };
+    const double per_guide = (double)text.n_bases * expected_hits_per_base(k, extra_pam);
+    const int rc = stream_ranges(n_guides, target, per_guide, scan, deliver, stats, err);
+    std::vector<std::thread> th;                      // the contexts go as for_each_shard's own do: one thread per device
+    for (vs_ctx *c : ctx) if (c) th.emplace_back([c] { vs_ctx_destroy(c); });
+    for (auto &t : th) t.join();
+    return rc;
 }
 
 }  // namespace vs
@@ -919,6 +1113,24 @@ struct vs_mapper {
     uint64_t planned_bytes = 0;
     std::atomic<bool> busy{false};
 };
+
+// the mapper's resident shards scan every guide range
+static int map_resident(vs_mapper *m, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam, uint64_t target, bool windows,
+                        const vs::RangeDeliver &deliver, vs_scan_stats *stats, std::string &err)
+{
+    const size_t n_shards = m->bounds.size() - 1;
+    const vs::RangeScan scan = [&](uint32_t lo, uint32_t hi, vs::RangeLists &lists, vs_scan_stats *st, std::string &e) {
+        vs::reset_lists(lists, n_shards);
+        return vs::for_each_shard(m->bounds, m->devices, &m->ctx, st, e, [&](int s, vs_ctx *ctx, uint64_t, uint64_t, vs_scan_stats *st1) {
+            uint64_t cnt = 0;
+            vs::Collect col{&lists.hits[(size_t)s], &lists.win[(size_t)s]};
+            return vs::scan_resolved_ex(ctx, nullptr, 0, 0, guides + (size_t)lo * VS_GLEN, hi - lo, k, extra_pam, nullptr, 0, &cnt, windows,
+                                        &vs::Collect::sink, &col, st1);
+        });
+    };
+    const double per_guide = (double)(m->bounds.back() * 32) * vs::expected_hits_per_base(k, extra_pam);
+    return vs::stream_ranges(n_guides, target, per_guide, scan, deliver, stats, err);
+}
 
 extern "C" void vs_mapper_destroy(vs_mapper *m)
 {
@@ -1014,14 +1226,32 @@ extern "C" int vs_mapper_map(vs_mapper *m, const uint8_t *guides, uint32_t n_gui
     bool idle = false;
     if (!m->busy.compare_exchange_strong(idle, true)) { vs_set_last_error("vs_mapper_map: one call at a time on a mapper"); return VS_ERR_ARG; }
     struct Release { std::atomic<bool> &b; ~Release() { b.store(false); } } release{m->busy};
-    std::vector<std::vector<vs_loc_hit>> lists(m->bounds.size() - 1);
     std::string err;
-    int rc = vs::for_each_shard(m->bounds, m->devices, &m->ctx, stats, err, [&](int s, vs_ctx *ctx, uint64_t, uint64_t, vs_scan_stats *st) {
-        uint64_t cnt = 0;
-        return vs_scan_resolved(ctx, nullptr, 0, 0, guides, n_guides, k, extra_pam, nullptr, 0, &cnt, &vs::append_sink, &lists[(size_t)s], st);
-    });
-    if (rc != VS_OK) { vs_set_last_error(("vs_mapper_map: " + err).c_str()); return rc; }
-    return vs::merge_lists(lists, n_threads, records, n_records, key16_collisions);
+    const int rc = map_resident(m, guides, n_guides, k, extra_pam, UINT64_MAX, false, vs::merge_all(n_threads, records, n_records, key16_collisions), stats, err);
+    if (rc != VS_OK) vs_set_last_error(("vs_mapper_map: " + err).c_str());
+    return rc;
+}
+
+extern "C" int vs_mapper_map_stream(vs_mapper *m, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam, int n_threads,
+                                    uint64_t records_per_delivery, int with_windows, vs_record_sink sink, void *user,
+                                    uint64_t *key16_collisions, vs_scan_stats *stats)
+{
+    if (key16_collisions) *key16_collisions = 0;
+    if (!m || !sink || (n_guides && !guides)) { vs_set_last_error("vs_mapper_map_stream: NULL argument"); return VS_ERR_ARG; }
+    if (const char *why = vs::scan_arg_error(guides, n_guides, k, extra_pam)) {
+        vs_set_last_error((std::string("vs_mapper_map_stream: ") + why).c_str());
+        return VS_ERR_ARG;
+    }
+    bool idle = false;
+    if (!m->busy.compare_exchange_strong(idle, true)) { vs_set_last_error("vs_mapper_map_stream: one call at a time on a mapper"); return VS_ERR_ARG; }
+    struct Release { std::atomic<bool> &b; ~Release() { b.store(false); } } release{m->busy};
+    const uint64_t target = records_per_delivery ? records_per_delivery : vs::DEFAULT_RECORDS_PER_DELIVERY;
+    vs::SinkDeliver d{target, with_windows != 0, n_threads, sink, user};
+    std::string err;
+    const int rc = map_resident(m, guides, n_guides, k, extra_pam, target, with_windows != 0, std::ref(d), stats, err);
+    if (key16_collisions) *key16_collisions = d.collisions;
+    if (rc != VS_OK) vs_set_last_error(("vs_mapper_map_stream: " + err).c_str());
+    return rc;
 }
 
 extern "C" int vs_mapper_info(const vs_mapper *m, uint32_t *n_shards, uint64_t *device_bytes, uint64_t *planned_bytes)
@@ -1071,11 +1301,32 @@ extern "C" int vs_map_records(const vs_text_view *text, const uint8_t *guides, u
     *records = nullptr; *n_records = 0;
     std::vector<int> dev;
     for (int i = 0; i < n_devices && devices; ++i) dev.push_back(devices[i]);
-    std::vector<std::vector<vs_loc_hit>> lists;
     std::string err;
-    int rc = vs::scan_text_sharded_resolved(*text, dev, guides, n_guides, k, extra_pam, lists, stats, err);
-    if (rc != VS_OK) { vs_set_last_error(err.c_str()); return rc; }
-    return vs::merge_lists(lists, n_threads, records, n_records, key16_collisions);
+    const int rc = vs::map_text(*text, dev, guides, n_guides, k, extra_pam, UINT64_MAX, false, vs::merge_all(n_threads, records, n_records, key16_collisions),
+                                stats, err);
+    if (rc != VS_OK) vs_set_last_error(err.c_str());
+    return rc;
+}
+
+extern "C" int vs_map_records_stream(const vs_text_view *text, const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
+                                     const int *devices, int n_devices, int n_threads, uint64_t records_per_delivery, int with_windows,
+                                     vs_record_sink sink, void *user, uint64_t *key16_collisions, vs_scan_stats *stats)
+{
+    if (key16_collisions) *key16_collisions = 0;
+    if (!text || !sink || (n_guides && !guides) || (n_devices > 0 && !devices)) { vs_set_last_error("vs_map_records_stream: NULL argument"); return VS_ERR_ARG; }
+    if (const char *why = vs::scan_arg_error(guides, n_guides, k, extra_pam)) {
+        vs_set_last_error((std::string("vs_map_records_stream: ") + why).c_str());
+        return VS_ERR_ARG;
+    }
+    std::vector<int> dev;
+    for (int i = 0; i < n_devices; ++i) dev.push_back(devices[i]);
+    const uint64_t target = records_per_delivery ? records_per_delivery : vs::DEFAULT_RECORDS_PER_DELIVERY;
+    vs::SinkDeliver d{target, with_windows != 0, n_threads, sink, user};
+    std::string err;
+    const int rc = vs::map_text(*text, dev, guides, n_guides, k, extra_pam, target, with_windows != 0, std::ref(d), stats, err);
+    if (key16_collisions) *key16_collisions = d.collisions;
+    if (rc != VS_OK) vs_set_last_error(("vs_map_records_stream: " + err).c_str());
+    return rc;
 }
 
 extern "C" int vs_shard_bounds(uint64_t n_words, int n_shards, uint64_t *out)

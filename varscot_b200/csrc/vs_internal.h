@@ -1,6 +1,7 @@
 // varscot_b200/csrc/vs_internal.h — helpers shared by the host and device halves of libvarscot_scan.
 #pragma once
 #include "../../include/varscot_scan.h"
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -22,11 +23,59 @@ int scan_text_sharded(const vs_text_view &text, const std::vector<int> &devices,
                       const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
                       std::vector<vs_hit> &hits, vs_scan_stats *agg, std::string &err);
 
-// The same with every shard's hits resolved to (contig, pos) and sorted on its device (vs_scan_resolved): one list per
-// shard, in shard order, ready for vs_merge_resolved.
-int scan_text_sharded_resolved(const vs_text_view &text, const std::vector<int> &devices,
-                               const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
-                               std::vector<std::vector<vs_loc_hit>> &lists, vs_scan_stats *agg, std::string &err);
+// vs_scan_resolved with the genome window of every hit (k_loc_windows) when `windows` is set: the sink receives each
+// super-chunk's sorted hits and, with windows, one uint64_t per hit (the format of vs_record_sink); NULL otherwise.
+typedef int (*loc_sink)(void *user, const vs_loc_hit *hits, const uint64_t *windows, uint64_t n, uint32_t guide_lo, uint32_t guide_hi);
+int scan_resolved_ex(vs_ctx *ctx, const vs_text_view *text, uint64_t first_word, uint64_t n_words,
+                     const uint8_t *guides, uint32_t n_guides, int k, int extra_pam,
+                     vs_loc_hit *out, uint64_t out_cap, uint64_t *n_hits, bool windows, loc_sink sink, void *user, vs_scan_stats *stats);
+
+// Expected hits per guide and text base on uniform-random text at k mismatches and the PAM set of extra_pam (what a scan
+// sizes its hit buffer with).
+double expected_hits_per_base(int k, int extra_pam);
+
+// ---- guide-range streaming (vs_mapper_map_stream, vs_map_records_stream, and with one unlimited range vs_mapper_map and
+// vs_map_records) ----
+// The sorted lists of one guide range, one per shard, as vs_scan_resolved delivers them: guide ids (info >> 8) relative to the
+// range's first guide; win[s] holds one window per hit of hits[s] when windows were asked for, and is empty otherwise.
+struct RangeLists {
+    std::vector<std::vector<vs_loc_hit>> hits;
+    std::vector<std::vector<uint64_t>> win;
+    uint64_t total() const;
+};
+// Scan guides [lo, hi) on every shard into `out` (cleared by the callee), counting into *stats; err names a failure.
+using RangeScan = std::function<int(uint32_t lo, uint32_t hi, RangeLists &out, vs_scan_stats *stats, std::string &err)>;
+// A scanned range handed to the host: called on the calling thread, ranges in ascending order.  A code other than VS_OK stops
+// the stream and is returned, with the reason in err.
+using RangeDeliver = std::function<int(const RangeLists &lists, uint32_t lo, uint32_t hi, std::string &err)>;
+// deliver_pieces: the sink returned non-zero
+constexpr int SINK_ABORTED = -1;
+
+// Default target of records per delivery (records_per_delivery == 0).
+constexpr uint64_t DEFAULT_RECORDS_PER_DELIVERY = 32ull << 20;
+
+// Guides of the next range: target / the expected hits per guide (the last range's hits per guide once one was scanned),
+// at least 1, at most `left`.  target == UINT64_MAX: all of them.
+uint32_t next_range_guides(uint64_t target, double per_guide, uint32_t left);
+
+// The streaming driver: guide ranges [lo, hi) of whole guides in ascending order, sized by next_range_guides from
+// first_per_guide and then from each scanned range; while deliver() runs on range c on the calling thread, another thread
+// scans range c + 1 (a pipeline of depth two).  Stats are summed over the ranges.  Every thread is joined before it returns.
+int stream_ranges(uint32_t n_guides, uint64_t target, double first_per_guide, const RangeScan &scan, const RangeDeliver &deliver,
+                  vs_scan_stats *stats, std::string &err);
+
+// Merge of one range's lists (vs_merge_resolved) into records, guide ids offset by guide_base; with win_out, each record's window
+// travels through the same permutation.  Records of guides [g_lo, g_hi) (relative to the range) only.
+int merge_range(const RangeLists &lists, uint32_t g_lo, uint32_t g_hi, uint32_t guide_base, vs_record *out, uint64_t *win_out,
+                uint64_t *key16_collisions, int n_threads);
+// Records of guides [g_lo, g_hi) of the range (relative) in lists: sum over the shards.
+uint64_t range_count(const RangeLists &lists, uint32_t g_lo, uint32_t g_hi);
+
+// One range's deliveries to a vs_record_sink: split at guide borders into pieces of at most `target` records (a single guide
+// denser than that goes alone), each merged with guide ids offset by lo and handed to the sink; SINK_ABORTED when it returned
+// non-zero (no further call is made).  A range without records is one delivery with n = 0.
+int deliver_pieces(const RangeLists &lists, uint32_t lo, uint32_t hi, uint64_t target, bool windows, int n_threads,
+                   vs_record_sink sink, void *user, std::vector<vs_record> &rec, std::vector<uint64_t> &win, uint64_t *key16_collisions);
 
 // Split [0, n_words) into n contiguous shards of (almost) equal size, tile-aligned.
 std::vector<uint64_t> shard_bounds(uint64_t n_words, int n);

@@ -777,6 +777,36 @@ k_pack_loc_hits(const unsigned long long *__restrict__ keys, const unsigned long
     out[i] = r;
 }
 
+// 23 bits -> the even bits of a 64-bit word (bit i -> bit 2 i)
+__host__ __device__ __forceinline__ uint64_t spread_even(uint32_t x)
+{
+    uint64_t v = x & 0x7FFFFFu;
+    v = (v | (v << 16)) & 0x0000FFFF0000FFFFull;
+    v = (v | (v << 8)) & 0x00FF00FF00FF00FFull;
+    v = (v | (v << 4)) & 0x0F0F0F0F0F0F0F0Full;
+    v = (v | (v << 2)) & 0x3333333333333333ull;
+    v = (v | (v << 1)) & 0x5555555555555555ull;
+    return v;
+}
+
+// k_loc_windows: the genome window of every sorted hit.  The window start is rebuilt as k_resolve_hits defines it (the contig's
+// start + the position in the contig, modulo 2^32: the first contig may begin before the origin) and read from the resident
+// bases, whose word 0 sits at global_base (relative to the origin, as k_extract's); a window may end in the halo word.
+//   out[i] bits 2 j .. 2 j + 1 = Dna code (hi << 1 | lo) of genome base start + j, forward orientation (hits never hold an N)
+__global__ void __launch_bounds__(256)
+k_loc_windows(const vs_loc_hit *__restrict__ hits, uint64_t n, const uint32_t *__restrict__ starts, uint32_t first_contig,
+              const vs_bases *__restrict__ B, uint64_t global_base, uint64_t *__restrict__ out)
+{
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const vs_loc_hit h = hits[i];
+    const uint32_t start = starts[h.contig - first_contig] + (uint32_t)h.key;
+    const uint64_t p = (uint64_t)start - global_base;
+    const vs_bases a = B[p >> 5], b = B[(p >> 5) + 1];
+    const uint32_t s = (uint32_t)(p & 31);
+    out[i] = spread_even(__funnelshift_r(a.lo, b.lo, s)) | (spread_even(__funnelshift_r(a.hi, b.hi, s)) << 1);
+}
+
 #include "vs_bucket.cuh"
 
 // ------------------------------------------------------------------------------------------------

@@ -401,6 +401,59 @@ def map_records(text: PackedText, guides: np.ndarray, k: int, pam=None, devices=
     return rec, int(coll.value), st
 
 
+def _record_sink(sink, windows: bool):
+    """A RECORD_SINK that hands every delivery to sink(records REC_DT view, windows uint64 view or None, guide_lo, guide_hi) and
+    aborts the stream when it returns a truthy value.  An exception in sink aborts the stream too and is kept in .error."""
+    state = {"error": None}
+
+    def _cb(_user, rp, wp, n, lo, hi):
+        try:
+            if n:
+                rec = np.ctypeslib.as_array(C.cast(rp, C.POINTER(C.c_uint8)), shape=(n * REC_DT.itemsize,)).view(REC_DT)
+                win = np.ctypeslib.as_array(C.cast(wp, C.POINTER(C.c_uint64)), shape=(n,)) if windows else None
+            else:
+                rec, win = np.zeros(0, REC_DT), (np.zeros(0, np.uint64) if windows else None)
+            return 1 if sink(rec, win, lo, hi) else 0
+        except BaseException as e:      # noqa: BLE001  (re-raised by the caller once the library has returned)
+            state["error"] = e
+            return 1
+
+    return _lib.RECORD_SINK(_cb), state
+
+
+def _finish_stream(rc, state, coll, st):
+    if state["error"] is not None:
+        raise state["error"]
+    check(rc)
+    return int(coll.value), st
+
+
+def map_records_stream(text: PackedText, guides: np.ndarray, k: int, sink, pam=None, devices=None, threads: int = 1,
+                       records_per_delivery: int = 0, windows: bool = False):
+    """vs_map_records_stream: the records of map_records delivered a range of whole guides at a time, in emission order, while
+    the devices score the next range.  sink(records, windows, guide_lo, guide_hi) receives REC_DT and (with windows=True) uint64
+    views that are valid during the call only; a truthy return aborts (VarscotError VS_ERR_ARG).  records_per_delivery: target
+    records per delivery (0 = 32 Mi).  Returns (key16_collisions, stats)."""
+    L = _lib.lib()
+    g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
+    dev = np.asarray(devices if devices else [0], dtype=np.int32)
+    coll, st = C.c_uint64(), ScanStats()
+    cb, state = _record_sink(sink, windows)
+    v = text.view()
+    rc = L.vs_map_records_stream(C.byref(v), g.ctypes.data, g.shape[0], k, pam_code(pam) if not isinstance(pam, int) else pam,
+                                 dev.ctypes.data, len(dev), threads, records_per_delivery, int(bool(windows)), cb, None,
+                                 C.byref(coll), C.byref(st))
+    return _finish_stream(rc, state, coll, st)
+
+
+def md_from_window(window: int, guide: np.ndarray, strand: int, md_style: int = MD_SEQAN) -> str:
+    """vs_md_from_window: the MD:Z value of a delivered record from its genome window (what md_string gives for it)."""
+    buf = C.create_string_buffer(64)
+    g = np.ascontiguousarray(guide, dtype=np.uint8)
+    check(_lib.lib().vs_md_from_window(int(window), g.ctypes.data, strand, md_style, buf))
+    return buf.value.decode()
+
+
 class Mapper:
     """vs_mapper: map_records against a text kept resident in HBM.  The text is sharded over `devices` (default: device 0) as
     map_records shards it and uploaded once; every shard keeps its candidate indexes, so later calls with the same PAM set only
@@ -426,6 +479,17 @@ class Mapper:
         finally:
             self._L.vs_free(rp)
         return rec, int(coll.value), st
+
+    def map_stream(self, guides: np.ndarray, k: int, sink, pam=None, threads: int = 1, records_per_delivery: int = 0,
+                   windows: bool = False):
+        """vs_mapper_map_stream: map()'s records delivered a range of whole guides at a time (see map_records_stream).  Returns
+        (key16_collisions, stats)."""
+        g = np.ascontiguousarray(guides, dtype=np.uint8).reshape(-1, GLEN)
+        coll, st = C.c_uint64(), ScanStats()
+        cb, state = _record_sink(sink, windows)
+        rc = self._L.vs_mapper_map_stream(self._m, g.ctypes.data, g.shape[0], k, pam_code(pam) if not isinstance(pam, int) else pam,
+                                          threads, records_per_delivery, int(bool(windows)), cb, None, C.byref(coll), C.byref(st))
+        return _finish_stream(rc, state, coll, st)
 
     def _info(self):
         n, now, planned = C.c_uint32(), C.c_uint64(), C.c_uint64()
